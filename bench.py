@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B200 TTS tail (mel chunks -> HiFiGAN -> chunker -> 16k->8k -> G.711).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): concurrent real-time 8 kHz G.711 TTS streams per job at RTF <= 1
 = seconds of audio produced per second of device time.  A step is one reference `infer()` tail
@@ -33,6 +33,22 @@ FLOP_PER_WINDOW_ALL = 12 * 273.318e6 + 25.68e6 + 0.057e6 * 4
 # the three stages the fused ResBlock kernel covers (C = 128, 64, 32): 33.03 MMAC per frame per stage, algorithmic (no halo rows)
 FLOP_PER_WINDOW_RESBLOCK_STAGE = 12 * 2 * 33.030144e6
 CODEC_BYTES_PER_OUT = 9.0                                            # 2 fp32 in + 1 byte out per 8 kHz sample
+DUMP_BYTES = 60 << 20                                                # --dump-outputs: all files of one run together, under 64 MB with headers
+
+
+def dump_outputs(out_dir: str, arrays: dict, rank: int = 0, world: int = 1) -> None:
+    """Writes what the timed path returned in its last step as out_dir/<name>.npy (float32), so that two builds can be compared
+    output for output.  Each rank gets an equal share of DUMP_BYTES; an array larger than its share keeps a fixed, seeded sample
+    of its rows (sessions), in row order, so the same arguments select the same rows in every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // (len(arrays) * world)
+    for name, t in arrays.items():
+        a = t.cpu().numpy().astype(np.float32)
+        keep = max(1, share // max(a[0].nbytes, 1))
+        if a.shape[0] > keep:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}_rank{rank}.npy" if world > 1 else f"{name}.npy"), a)
 
 
 def load_peaks():
@@ -405,13 +421,15 @@ def main_b200(args, rank, local_rank, world):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        tail.tail(slots_d, mel_d, want_audio=False)
+        g711, _ = tail.tail(slots_d, mel_d, want_audio=False)
     e1.record()
     barrier()
     launches = kernel_launch_count() - l0
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     audio_s = S * world * F * AUDIO_S_PER_FRAME * args.steps
     value = audio_s / (ms_total / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"g711": g711}, rank, world)
 
     # ---- end-to-end timing with HOST buffers -----------------------------------------------------------
     # (a) the blocking C-ABI call (b2_tts_tail_host: H2D -> tail -> D2H -> sync, nothing overlapped): what a caller pays per call
@@ -625,7 +643,7 @@ def main_b200(args, rank, local_rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--sessions", type=int, default=1024, help="concurrent sessions per GPU")
@@ -644,7 +662,14 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling block (BASELINE config 3 as written)")
     ap.add_argument("--strong-total", type=int, default=1024)
     ap.add_argument("--cpu-sweep", action="store_true", help="with --impl reference: fp32/bf16 x B in {1,8,64} CPU table (SURVEY 8d)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU arm: after the timed steps, write the G.711 codes of the last timed step (sessions x samples) as DIR/g711.npy "
+                         "(float32, at most 64 MB; larger outputs keep a fixed, seeded sample of sessions)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
