@@ -169,7 +169,7 @@ B2_API int b2_sched_prebuild(b2_sched *s, int max_sessions);
  * Weights by state_dict key of transformers SpeechT5ForTextToSpeech: `speecht5.decoder.prenet.*`, `speecht5.decoder.wrapped_decoder.layers.*`,
  * `speech_decoder_postnet.feat_out.*`, `speech_decoder_postnet.prob_out.*`, plus key `pe` = the (max_steps, 768) position table
  * (SpeechT5ScaledPositionalEncoding.pe, modeling_speecht5.py:405-412; passed in so that it is torch's own).  Default SpeechT5Config sizes.
- * The text encoder (HelloSippyRTPipe.py:111-116, once per sentence) stays with the caller: its output is an input here.
+ * The text encoder's output (b2_enc_forward below, or any other encoder) is an input here.
  * B2_MODE_FP32: CUDA-core fp32 Linears, fp32 caches.  B2_MODE_BF16: tcgen05 GEMMs fed by TMA, bf16 caches, fp32 residual stream / LayerNorm. */
 typedef struct b2_dec b2_dec;
 /* max_rows: sessions per internal pass (workspace); max_steps: decoder steps a sentence may run (KV cache depth = positions of `pe`);
@@ -194,6 +194,29 @@ B2_API int b2_dec_get_step(b2_dec *dec, int slot, int32_t *h_step, void *stream)
 /* b2_dec_steps runs as ONE CUDA graph launch per call (cached per padded batch size and step count; a call is ~74 kernels per step).
  * on = 0 launches the kernels one by one instead (default: 1). */
 B2_API int b2_dec_set_graphs(b2_dec *dec, int on);
+
+/* ---- the text encoder (HelloSippyRTPipe.py:111-116, once per sentence): SpeechT5EncoderWithTextPrenet, token ids -> encoder_last_hidden_state ----
+ * prenet (embedding + alpha * scaled sinusoidal positions) -> LayerNorm -> twelve post-LN layers (self-attention with the relative-position
+ * term of SpeechT5RelativePositionalEncoding, GELU feed-forward), modeling_speecht5.py:765-781, :1013-1066, :1230-1320.
+ * Weights by state_dict key of transformers SpeechT5ForTextToSpeech: `speecht5.encoder.prenet.{embed_tokens.weight, encode_positions.alpha}`,
+ * `speecht5.encoder.wrapped_encoder.{layer_norm.*, embed_positions.pe_k.weight, layers.*}`, plus key `pe` = the (max_len, 768) position table
+ * (SpeechT5ScaledPositionalEncoding.pe, a non-persistent buffer: passed in so that it is torch's own).  Default SpeechT5Config sizes.
+ * Ragged: only valid tokens are computed; the sentences of a call are packed into passes of <= max_tokens rows (a sentence is never split),
+ * and a sentence's output does not depend on its companions or on the packing.
+ * B2_MODE_FP32: CUDA-core fp32 Linears.  B2_MODE_BF16: tcgen05 GEMMs fed by TMA; fp32 residual stream, LayerNorm and attention. */
+typedef struct b2_enc b2_enc;
+/* max_tokens: rows of one internal pass (workspace); max_len: positions per sentence, <= 450 (the scaled positional table) */
+B2_API b2_enc *b2_enc_create(int device, int mode, int max_tokens, int max_len);
+B2_API void b2_enc_destroy(b2_enc *enc);
+B2_API size_t b2_enc_device_bytes(const b2_enc *enc);
+B2_API int b2_enc_load_tensor(b2_enc *enc, const char *key, const float *h_data, const int64_t *shape, int ndim);  /* + key "pe" (max_len, 768) */
+B2_API int b2_enc_finalize(b2_enc *enc);
+/* d_ids (n, L) int32 device, right-padded; h_len (n) HOST valid lengths in [1, L] (NULL: all L); d_out (n, L, 768) fp32 device =
+ * encoder_last_hidden_state at valid positions, zeros elsewhere.  Only valid tokens are computed; sessions are packed into passes of
+ * <= max_tokens rows (a session is never split).  Asynchronous on `stream`.  Calls on one handle must be ordered (one stream). */
+B2_API int b2_enc_forward(b2_enc *enc, const int32_t *d_ids, const int32_t *h_len, int n, int L, float *d_out, void *stream);
+/* token ids outside [0, 81) are embedded as zeros and flagged; reported here (stream synchronised) or by the next call */
+B2_API int b2_enc_poll_errors(b2_enc *enc, void *stream);
 
 /* ---- Core/Codecs (G711.py:25-47), ctx-less, stateless ----------------------------------------------- */
 /* G711Codec.encode: clamp(x*32767,-32768,32767) -> int16 (trunc toward zero) -> G.711 code.  n samples. */

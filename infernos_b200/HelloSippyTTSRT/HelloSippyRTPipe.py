@@ -22,8 +22,9 @@ What differs, by design:
     (`postnet_state_dict`, or automatically when the engine loads a SpeechT5 model itself); `frontend.postnet` is then not called.
   * the autoregressive front half is reached through a small `frontend` object.  B200Frontend (SURVEY section 8 f3) runs the decoder loop of
     :195-229 -- prenet, six decoder layers with a slot KV cache, feat_out / prob_out, 16 steps per engine call -- inside the CUDA library
-    (engine.TTSDecoder, b2_dec_*) and hands the frames to the tail without leaving the device; the tokenizer and the text encoder (:111-116,
-    once per sentence) are two callables.  SpeechT5Frontend issues the reference's own torch calls on a transformers model; ScriptedFrontend
+    (engine.TTSDecoder, b2_dec_*) and hands the frames to the tail without leaving the device.  The text encoder (:111-116, once per
+    sentence) is a callable: engine.TTSEncoder (b2_enc_*, ragged: padded positions are never computed) with B200Frontend.from_state_dict or
+    from_model(gpu_encoder=True), the transformers model's own encoder otherwise; the tokenizer is a host callable.  SpeechT5Frontend issues the reference's own torch calls on a transformers model; ScriptedFrontend
     replays a fixed mel plan (tests, benchmarks of the tail alone).
   * requests may ask for pre-encoded dispatch (`pre_encoded=True`): `dispatch` then receives G711AudioChunk objects (samples + the G.711 bytes
     made on the GPU in the same pass), which the payload-aware OutputMuxer carries to the RTP packetiser un-re-encoded (f1).
@@ -226,10 +227,11 @@ class SpeechT5Frontend:
 class B200Frontend:
     """The autoregressive front half on the GPU (SURVEY section 8 f3): prenet -> six-layer decoder with a slot KV cache -> feat_out /
     prob_out run inside the CUDA library (engine.TTSDecoder, b2_dec_*), 16 steps per engine call in one C-ABI call, and the frames never leave
-    the device on their way into the tail.  What stays outside is what the reference runs once per sentence: the tokenizer and the text
-    encoder (:111-116), reached through two callables:
-        tokenizer(text) -> (1, n) LongTensor          (default: the SpeechT5 processor of `model`)
-        encoder(input_ids, attention_mask) -> (B, L, 768) tensor     (default: model.speecht5.encoder(...).last_hidden_state)
+    the device on their way into the tail.  What the reference runs once per sentence (:111-116) is reached through two callables:
+        tokenizer(text) -> (1, n) LongTensor          (the SpeechT5 processor with from_model; any callable with from_state_dict)
+        encoder(input_ids, attention_mask) -> (B, L, 768) tensor
+    The encoder is engine.TTSEncoder -- the text encoder inside the library, only valid tokens computed -- with from_state_dict() and with
+    from_model(gpu_encoder=True); from_model() without it keeps model.speecht5.encoder(...).last_hidden_state on the transformers model.
     `mask_fn(call_index) -> (16, 2, 256) 0/1 tensor` injects the prenet's dropout keep-masks (tests); by default they are drawn on the device."""
 
     reduction_factor = 2
@@ -240,15 +242,41 @@ class B200Frontend:
         self.decoder, self._tokenize, self._encode, self.mask_fn, self.seed = decoder, tokenizer, encoder, mask_fn, seed
 
     @classmethod
-    def from_model(cls, model, processor, device, mode="bf16", max_sessions=64, max_steps=512, max_enc_len=128, **kw):
-        from infernos_b200.engine import TTSDecoder
-        dec = TTSDecoder(device, model.state_dict(), mode=mode, max_sessions=max_sessions, max_steps=max_steps, max_enc_len=max_enc_len)
-
-        @torch.no_grad()
-        def encode(ids, mask):
-            dev = next(model.parameters()).device
-            return model.speecht5.encoder(input_values=ids.to(dev), attention_mask=mask.to(dev), return_dict=True).last_hidden_state
+    def from_model(cls, model, processor, device, mode="bf16", max_sessions=64, max_steps=512, max_enc_len=128, gpu_encoder=False,
+                   max_tokens=16384, **kw):
+        """gpu_encoder=True runs the text encoder in the library too (engine.TTSEncoder on the model's weights); the default keeps the model's
+        own torch encoder."""
+        from infernos_b200.engine import TTSDecoder, TTSEncoder
+        sd = model.state_dict()
+        dec = TTSDecoder(device, sd, mode=mode, max_sessions=max_sessions, max_steps=max_steps, max_enc_len=max_enc_len)
+        if gpu_encoder:
+            encode = TTSEncoder(device, sd, mode=mode, max_tokens=max_tokens, max_len=max_enc_len)
+        else:
+            @torch.no_grad()
+            def encode(ids, mask):
+                dev = next(model.parameters()).device
+                return model.speecht5.encoder(input_values=ids.to(dev), attention_mask=mask.to(dev), return_dict=True).last_hidden_state
         return cls(dec, lambda text: processor(text=text, return_tensors="pt")["input_ids"], encode, **kw)
+
+    @classmethod
+    def from_state_dict(cls, sd, tokenizer: Callable, device, mode="bf16", max_sessions=64, max_steps=512, max_enc_len=128, max_tokens=16384, **kw):
+        """Token ids to frames without a transformers model object: engine.TTSEncoder and engine.TTSDecoder built from one SpeechT5ForTextToSpeech
+        state_dict (`speecht5.encoder.*`, `speecht5.decoder.*`, `speech_decoder_postnet.{feat_out,prob_out}.*`).  max_enc_len (<= 450) bounds
+        the padded token length of a cohort; max_tokens the rows of one encoder pass."""
+        from infernos_b200.engine import TTSDecoder, TTSEncoder
+        dec = TTSDecoder(device, sd, mode=mode, max_sessions=max_sessions, max_steps=max_steps, max_enc_len=max_enc_len)
+        try:
+            enc = TTSEncoder(device, sd, mode=mode, max_tokens=max_tokens, max_len=max_enc_len)
+        except Exception:
+            dec.close()
+            raise
+        return cls(dec, tokenizer, enc, **kw)
+
+    def close(self) -> None:
+        """Frees the library handles this front half owns (the decoder, and the encoder when it is an engine.TTSEncoder)."""
+        self.decoder.close()
+        if hasattr(self._encode, "close"):
+            self._encode.close()
 
     def tokenize(self, text):
         return self._tokenize(text)

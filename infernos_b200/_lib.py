@@ -57,6 +57,13 @@ SIGNATURES = {
     "b2_dec_poll_errors": (c_int, [c_void_p, c_void_p]),
     "b2_dec_set_graphs": (c_int, [c_void_p, c_int]),
     "b2_dec_get_step": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
+    "b2_enc_create": (c_void_p, [c_int, c_int, c_int, c_int]),
+    "b2_enc_destroy": (None, [c_void_p]),
+    "b2_enc_device_bytes": (c_size_t, [c_void_p]),
+    "b2_enc_load_tensor": (c_int, [c_void_p, c_char_p, c_void_p, POINTER(c_int64), c_int]),
+    "b2_enc_finalize": (c_int, [c_void_p]),
+    "b2_enc_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "b2_enc_poll_errors": (c_int, [c_void_p, c_void_p]),
     "b2_session_reset": (c_int, [c_void_p, c_void_p, c_int, c_void_p]),
     "b2_session_get_pre_frames": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "b2_session_set_pre_frames": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),

@@ -439,6 +439,91 @@ class TTSDecoder:
         return int(v.value)
 
 
+ENCODER_TENSORS = 2 + 2 + 1 + 12 * 16       # prenet (embedding, alpha), first LayerNorm, pe_k, 12 layers x 16
+
+
+class TTSEncoder:
+    """The SpeechT5 text encoder on the GPU (b2_enc_*): token ids -> encoder_last_hidden_state, what the reference runs once per sentence
+    (HelloSippyRTPipe.py:111-116).  `sd` is a state_dict that holds the `speecht5.encoder.*` tensors of transformers SpeechT5ForTextToSpeech
+    (the whole model's state_dict will do).  Only the valid tokens of a batch are computed: sentences are packed back to back into passes
+    of at most `max_tokens` rows; `max_len` (<= 450, the model's max_text_positions) bounds the padded length of a call."""
+
+    def __init__(self, device, sd: Dict[str, torch.Tensor], mode="bf16", max_tokens: int = 16384, max_len: int = 450):
+        self.lib = _lib.load()
+        self.device = torch.device(device)
+        if self.device.type != "cuda" or not torch.cuda.is_available():
+            raise RuntimeError("infernos_b200 runs on CUDA devices only (no CPU fallback)")
+        self.index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        self.device = torch.device("cuda", self.index)
+        self.mode = _MODES[mode]
+        self.max_tokens, self.max_len = int(max_tokens), int(max_len)
+        self.h = self.lib.b2_enc_create(self.index, self.mode, self.max_tokens, self.max_len)
+        if not self.h:
+            raise RuntimeError("b2_enc_create: " + self.lib.b2_last_error(None).decode())
+        try:
+            n = 0
+            for k, v in sd.items():
+                if not k.startswith("speecht5.encoder.") or k.endswith("encode_positions.pe"):
+                    continue
+                self._load(k, v)
+                n += 1
+            if n != ENCODER_TENSORS:
+                raise RuntimeError(f"encoder state_dict: expected {ENCODER_TENSORS} tensors, found {n}")
+            self._load("pe", decoder_position_table(self.max_len))
+            with torch.cuda.device(self.index):
+                _lib.check(self.lib.b2_enc_finalize(self.h), "enc_finalize")
+        except Exception:
+            self.close()
+            raise
+
+    def _load(self, k, v):
+        t = v.detach().to("cpu", torch.float32).contiguous()
+        shape = (ctypes.c_int64 * max(1, t.dim()))(*t.shape)
+        _lib.check(self.lib.b2_enc_load_tensor(self.h, k.encode(), ctypes.c_void_p(t.data_ptr()), shape, t.dim()), f"enc load {k}")
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.lib.b2_enc_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def device_bytes(self) -> int:
+        return int(self.lib.b2_enc_device_bytes(self.h))
+
+    def __call__(self, input_ids: torch.Tensor, attention_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """input_ids (B, L) integer (host or device), attention_mask (B, L) 0/1 with every row a prefix of ones (right padding) or None ->
+        (B, L, 768) fp32 on this device: encoder_last_hidden_state at valid positions, zeros at padded ones.  The `encoder` callable of
+        B200Frontend."""
+        if input_ids.dim() != 2:
+            raise RuntimeError("input_ids must be (B, L)")
+        B, L = input_ids.shape
+        lens = None
+        if attention_mask is not None:
+            m = attention_mask.detach().to("cpu", torch.int32)
+            if tuple(m.shape) != (B, L):
+                raise RuntimeError(f"attention_mask {tuple(m.shape)} does not match input_ids {(B, L)}")
+            lens = m.sum(1, dtype=torch.int32).contiguous()
+            if not torch.equal(m, (torch.arange(L)[None] < lens[:, None]).to(torch.int32)):
+                raise RuntimeError("attention_mask must be a prefix of ones in every row (right-padded sentences)")
+        ids = input_ids.to(device=self.device, dtype=torch.int32).contiguous()
+        out = torch.empty(B, L, 768, device=self.device, dtype=torch.float32)
+        with torch.cuda.device(self.index):
+            _lib.check(self.lib.b2_enc_forward(self.h, ids.data_ptr(), lens.data_ptr() if lens is not None else None, B, L, out.data_ptr(),
+                                               _stream_ptr(self.device)), "enc_forward")
+        return out
+
+    def poll_errors(self) -> None:
+        """Synchronises the current stream and raises if an earlier call was given token ids outside [0, 81)."""
+        with torch.cuda.device(self.index):
+            _lib.check(self.lib.b2_enc_poll_errors(self.h, _stream_ptr(self.device)), "enc_poll_errors")
+
+
 def postnet_layers(sd: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
     """Picks the post-net's conv / batch-norm tensors out of a SpeechT5 state_dict, whatever prefix they carry
     (`layers.0.conv.weight`, `speech_decoder_postnet.layers.0.conv.weight`, ...)."""

@@ -181,3 +181,52 @@ def synth_encoder_states(batch: int, length: int, seed: int = 99) -> torch.Tenso
 def synth_speakers(batch: int, seed: int = 98) -> torch.Tensor:
     g = torch.Generator().manual_seed(seed)
     return torch.randn(batch, DEC_SPK_DIM, generator=g) * 3.0
+
+
+ENCODER_SEED = 2029
+ENC_LAYERS, ENC_VOCAB, ENC_MAX_REL = 12, 81, 160
+# Gains of the random text encoder.  q / k at 1.4 / sqrt(fan_in) and pe_k rows at std 1.4 put both terms of the attention score (q.k and the
+# relative-position term q.pe_k, each with the 1/8-scaled q) at a spread of about 2: the softmax is far from uniform, and a sign or clamp error
+# in the relative positions changes the output at O(1).  The post-LN layers keep the residual stream at unit scale whatever the gains.
+G_ENC_QK, G_ENC_PEK, G_ENC_FFN1 = 1.4, 1.4, 1.4
+
+
+def encoder_state_dict(seed: int = ENCODER_SEED) -> Dict[str, torch.Tensor]:
+    """Random weights with the `speecht5.encoder.*` state_dict keys of transformers SpeechT5ForTextToSpeech (SpeechT5EncoderWithTextPrenet,
+    default SpeechT5Config: vocab 81, hidden 768, 12 layers, 12 heads, FFN 3072, relative positions +-160; modeling_speecht5.py:765-781,
+    1013-1066, 1230-1320), fp32, CPU.  The sinusoidal table `prenet.encode_positions.pe` is a non-persistent buffer and is not included."""
+    g = torch.Generator().manual_seed(seed)
+
+    def lin(cout, cin, gain=1.0):
+        return torch.randn(cout, cin, generator=g) * (gain / math.sqrt(cin))
+
+    sd: Dict[str, torch.Tensor] = {}
+    P, W = "speecht5.encoder.prenet.", "speecht5.encoder.wrapped_encoder."
+    sd[P + "embed_tokens.weight"] = torch.randn(ENC_VOCAB, DEC_HIDDEN, generator=g)
+    sd[P + "encode_positions.alpha"] = torch.tensor(0.8)
+    sd[W + "layer_norm.weight"] = torch.rand(DEC_HIDDEN, generator=g) * 0.4 + 0.8
+    sd[W + "layer_norm.bias"] = _bias(g, DEC_HIDDEN) * 5
+    sd[W + "embed_positions.pe_k.weight"] = torch.randn(2 * ENC_MAX_REL, DEC_HIDDEN // DEC_HEADS, generator=g) * G_ENC_PEK
+    for i in range(ENC_LAYERS):
+        L = W + f"layers.{i}."
+        for pj in ("k_proj", "v_proj", "q_proj", "out_proj"):
+            sd[L + f"attention.{pj}.weight"] = lin(DEC_HIDDEN, DEC_HIDDEN, G_ENC_QK if pj in ("q_proj", "k_proj") else 1.0)
+            sd[L + f"attention.{pj}.bias"] = _bias(g, DEC_HIDDEN)
+        sd[L + "layer_norm.weight"] = torch.rand(DEC_HIDDEN, generator=g) * 0.4 + 0.8
+        sd[L + "layer_norm.bias"] = _bias(g, DEC_HIDDEN) * 5
+        sd[L + "feed_forward.intermediate_dense.weight"] = lin(DEC_FFN, DEC_HIDDEN, G_ENC_FFN1)
+        sd[L + "feed_forward.intermediate_dense.bias"] = _bias(g, DEC_FFN)
+        sd[L + "feed_forward.output_dense.weight"] = lin(DEC_HIDDEN, DEC_FFN, 1.0)
+        sd[L + "feed_forward.output_dense.bias"] = _bias(g, DEC_HIDDEN)
+        sd[L + "final_layer_norm.weight"] = torch.rand(DEC_HIDDEN, generator=g) * 0.4 + 0.8
+        sd[L + "final_layer_norm.bias"] = _bias(g, DEC_HIDDEN) * 5
+    return sd
+
+
+def synth_token_ids(lengths, seed: int = 97) -> tuple:
+    """Right-padded token ids (B, max(lengths)) int64 in [4, 81) (0..3 are the tokenizer's special ids) and the matching 0/1 attention mask."""
+    g = torch.Generator().manual_seed(seed)
+    L = max(lengths)
+    ids = torch.randint(4, ENC_VOCAB, (len(lengths), L), generator=g)
+    mask = (torch.arange(L)[None] < torch.tensor(list(lengths))[:, None]).to(torch.int)
+    return ids * mask + (1 - mask), mask               # padding id 1 (SpeechT5's pad_token_id)
