@@ -251,6 +251,14 @@ B2_API int b2_conv1d_tc(const void *d_in_bf16, const float *h_weight, const floa
                         const float *d_residual, float *d_out32, void *d_outb, float slope, float div, void *stream);
 B2_API int b2_conv1d_f32(const float *d_in, const float *h_weight, const float *h_bias, int W, int T, int Cin, int Cout, int k, int dil,
                          float pre_slope, const float *d_residual, float *d_out32, void *d_outb, float slope, float div, void *stream);
+/* One Linear of the text encoder / speech decoder, C = act(A W^T + b) * colscale, through the same packing and launch (tile choice included)
+ * their passes use.  mode B2_MODE_BF16: d_in bf16 [a_rows][K], tcgen05 GEMM, d_out32 fp32 [M][N] and/or d_outb bf16 [M][N];
+ * B2_MODE_FP32: d_in fp32 [M][K], CUDA-core kernel, d_out32 only.  h_weight [N][K] and h_bias [N] host fp32 (torch layout); d_colscale [N]
+ * or NULL; act 0/1/2 = none / ReLU / GELU (erf).  a_rows >= M: rows the A tensor map spans (the encoder's and decoder's maps span their
+ * workspace, not the pass).  h_launched (may be NULL) receives {tile N, ring stages} of the launch ({0, 0} in fp32 mode).
+ * K and N multiples of 64; M = 0 does nothing.  Synchronous on `stream`. */
+B2_API int b2_linear(int device, int mode, const void *d_in, int M, int a_rows, const float *h_weight, const float *h_bias, int N, int K,
+                     int act, const float *d_colscale, float *d_out32, void *d_outb, int *h_launched, void *stream);
 
 /* One whole HiFiGAN ResBlock (modeling_speecht5.py:2903-2962) in a single fused tcgen05 launch:
  *   for d in (d0, d1, d2): x = x + conv2(lrelu(conv1_dil_d(lrelu(x, slope)), slope));   v = (d_acc + x) / div

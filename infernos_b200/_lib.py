@@ -79,6 +79,8 @@ SIGNATURES = {
     "b2_g711_decode_many_host": (c_int, [c_void_p, c_void_p, c_size_t, c_int, c_int, c_void_p, c_void_p]),
     "b2_conv1d_tc": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_float, c_float, c_void_p]),
     "b2_conv1d_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_float, c_float, c_void_p]),
+    "b2_linear": (c_int, [c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                          POINTER(c_int), c_void_p]),
     "b2_resblock_tc": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                c_float, c_float, c_float, c_void_p]),
     "b2_resblock_t_plan": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int)]),

@@ -516,16 +516,21 @@ int make_tma_2d_bf16(CUtensorMap *tm, const void *ptr, long long rows, int K, lo
 
 static bool g_gemm_attr[64][5] = {};
 
+// ring depth: deep (8 x 24 KB / 6 x 32 KB) when the K loop is long enough to use it, 4 otherwise (B2_GEMM_DEEP=0: always 4)
+int gemm_tc_stages(int K, int nt) {
+    static const bool deep_on = !(getenv("B2_GEMM_DEEP") && atoi(getenv("B2_GEMM_DEEP")) == 0);
+    const bool deep = deep_on && K >= 512 && nt != 256;                 // 128 x 256 tiles: 4 x 48 KB is all the shared memory there is
+    return deep ? (nt == 128 ? 6 : 8) : 4;
+}
+
 int launch_gemm_tc(const GemmTcArgs &a, cudaStream_t st) {
     if (a.M <= 0) return 0;
     if (!a.tmA || !a.tmB || !a.bias || (a.nt != 64 && a.nt != 128 && a.nt != 256) || a.N % a.nt || a.K % 64 || a.K < 64) return set_error("gemm_tc: bad arguments (N %d nt %d K %d)", a.N, a.nt, a.K);
     GemmParams p;
     p.bias = a.bias; p.colscale = a.colscale; p.out32 = a.out32; p.outb = a.outb; p.M = a.M; p.N = a.N; p.K = a.K; p.ldo = a.N; p.act = a.act;
     dim3 grid((unsigned)cdiv(a.M, 128), (unsigned)(a.N / a.nt));
-    // ring depth: deep (8 x 24 KB / 6 x 32 KB) when the K loop is long enough to use it, 4 otherwise (B2_GEMM_DEEP=0: always 4)
-    static const bool deep_on = !(getenv("B2_GEMM_DEEP") && atoi(getenv("B2_GEMM_DEEP")) == 0);
-    const bool deep = deep_on && a.K >= 512 && a.nt != 256;             // 128 x 256 tiles: 4 x 48 KB is all the shared memory there is
-    const int stages = deep ? (a.nt == 128 ? 6 : 8) : 4;
+    const int stages = gemm_tc_stages(a.K, a.nt);
+    const bool deep = stages != 4;
     const int slot = a.nt == 256 ? 4 : (a.nt == 128 ? 1 : 0) + (deep ? 2 : 0);
     const size_t smem = (size_t)stages * (128 * 64 * 2 + (size_t)a.nt * 64 * 2) + (2 * stages + 1) * 8 + 16;
     int dev = 0;
@@ -901,6 +906,36 @@ int b2_dec_get_step(b2_dec *d, int slot, int32_t *h_step, void *stream) {
     B2_CUDA_OK(cudaMemcpyAsync(h_step, d->step + slot, sizeof(int32_t), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     B2_CUDA_OK(cudaStreamSynchronize((cudaStream_t)stream));
     return 0;
+}
+
+int b2_linear(int device, int mode, const void *d_in, int M, int a_rows, const float *h_weight, const float *h_bias, int N, int K, int act,
+              const float *d_colscale, float *d_out32, void *d_outb, int *h_launched, void *stream) {
+    if (mode != B2_MODE_FP32 && mode != B2_MODE_BF16) return set_error("b2_linear: mode must be B2_MODE_FP32 or B2_MODE_BF16");
+    if (M < 0 || a_rows < M || K < 64 || K % 64 || N < 64 || N % 64 || act < 0 || act > 2)
+        return set_error("b2_linear: bad arguments (M %d a_rows %d N %d K %d act %d; need a_rows >= M, K and N multiples of 64, act 0..2)", M, a_rows, N, K, act);
+    if (mode == B2_MODE_FP32 && (d_outb || !d_out32)) return set_error("b2_linear: fp32 mode writes d_out32 only");
+    if (h_launched) h_launched[0] = h_launched[1] = 0;
+    if (M == 0) return 0;
+    if (!d_in || !h_weight || !h_bias || (!d_out32 && !d_outb)) return set_error("b2_linear: null pointer");
+    B2_CUDA_OK(cudaSetDevice(device));
+    cudaStream_t st = (cudaStream_t)stream;
+    LinearOwner o;
+    o.what = "b2_linear"; o.device = device; o.mode = mode; o.use_pdl = pdl_enabled();
+    DecLinear l;
+    std::vector<float> W(h_weight, h_weight + (size_t)N * K), B(h_bias, h_bias + N);
+    CUtensorMap tmA;
+    int rc = mode == B2_MODE_BF16 ? get_encoder() : 0;
+    if (!rc) rc = upload_linear(&o, l, K, N, W, B);
+    if (!rc && mode == B2_MODE_BF16) rc = make_map(&tmA, d_in, a_rows, K, 128);
+    if (!rc) rc = linear(&o, l, static_cast<const float *>(d_in), &tmA, M, act, d_colscale, d_out32, static_cast<__nv_bfloat16 *>(d_outb), st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (!rc && e != cudaSuccess) rc = set_error("b2_linear: %s", cudaGetErrorString(e));
+    if (!rc && h_launched && mode == B2_MODE_BF16) {
+        h_launched[0] = gemm_tile_n(l, M);
+        h_launched[1] = gemm_tc_stages(K, h_launched[0]);
+    }
+    for (void *p : o.allocs) cudaFree(p);
+    return rc;
 }
 
 }  // extern "C"

@@ -16,6 +16,8 @@ struct GemmTcArgs {
     bool pdl = false;                   // launch with the programmatic-stream-serialization attribute (the decoder's kernel chain)
 };
 int launch_gemm_tc(const GemmTcArgs &a, cudaStream_t st);
+// stages of the shared-memory operand ring launch_gemm_tc uses for K and tile width nt
+int gemm_tc_stages(int K, int nt);
 // TMA map over row-major bf16 [rows][K] with `row_stride` ELEMENTS between rows (>= K), box 64 x box_rows, 128-byte swizzle
 int make_tma_2d_bf16(CUtensorMap *tm, const void *ptr, long long rows, int K, long long row_stride, int box_rows);
 

@@ -179,6 +179,14 @@ inline int upload_vec(LinearOwner *d, float **dst, const HostTensor &t) {
     return 0;
 }
 
+// Tile width of a bf16-mode Linear's GEMM over M rows.  One tile per CTA: when the 128 x 128 tiles of a wide layer do not fit one wave (ffn1 at
+// 1,024 rows: 8 x 24 = 192 CTAs on 148 SMs, the second wave 30 % full: 46 us against 21 us for the 144-CTA qkv GEMM), 128 x 256 tiles do (96 CTAs).
+// B2_GEMM_NT256=0 keeps 128.
+inline int gemm_tile_n(const DecLinear &l, int M) {
+    static const bool nt256_on = !(getenv("B2_GEMM_NT256") && atoi(getenv("B2_GEMM_NT256")) == 0);
+    return nt256_on && l.has256 && (long long)cdiv(M, 128) * (l.N / 128) > sm_count() ? 256 : l.nt;
+}
+
 // C = act(A W^T + bias) * colscale.  fp32 mode: A32 [M][K] through the CUDA-core conv kernel (+ k_act_scale); bf16 mode: tmA over the bf16 A buffer.
 inline int linear(LinearOwner *d, const DecLinear &l, const float *A32, const CUtensorMap *tmA, int M, int act, const float *colscale,
                   float *out32, __nv_bfloat16 *outb, cudaStream_t st) {
@@ -186,11 +194,9 @@ inline int linear(LinearOwner *d, const DecLinear &l, const float *A32, const CU
     if (M <= 0) return 0;
     if (d->mode == B2_MODE_BF16) {
         GemmTcArgs g;
-        g.tmA = tmA; g.tmB = &l.tmB; g.bias = l.bias; g.colscale = colscale; g.out32 = out32; g.outb = outb; g.M = M; g.N = l.N; g.K = l.K; g.nt = l.nt; g.act = act; g.pdl = d->use_pdl;
-        // One tile per CTA: when the 128 x 128 tiles of a wide layer do not fit one wave (ffn1 at 1,024 rows: 8 x 24 = 192 CTAs on 148 SMs, the second
-        // wave 30 % full: 46 us against 21 us for the 144-CTA qkv GEMM), 128 x 256 tiles do (96 CTAs).  B2_GEMM_NT256=0 keeps 128.
-        static const bool nt256_on = !(getenv("B2_GEMM_NT256") && atoi(getenv("B2_GEMM_NT256")) == 0);
-        if (nt256_on && l.has256 && (long long)cdiv(M, 128) * (l.N / 128) > sm_count()) { g.tmB = &l.tmB256; g.nt = 256; }
+        g.tmA = tmA; g.bias = l.bias; g.colscale = colscale; g.out32 = out32; g.outb = outb; g.M = M; g.N = l.N; g.K = l.K; g.act = act; g.pdl = d->use_pdl;
+        g.nt = gemm_tile_n(l, M);
+        g.tmB = g.nt == 256 ? &l.tmB256 : &l.tmB;
         return launch_gemm_tc(g, st);
     }
     ConvArgs a;

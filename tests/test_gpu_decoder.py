@@ -217,3 +217,71 @@ def test_worker_with_gpu_front_half_reference_load_test_shape():
     # maxlen = 24 decoder steps -> ends_at = 26 -> (26 - 1) * 256 samples at 8 kHz
     assert abs(r["audio_s_per_session"] - 25 * 256 / 8000.0) < 1e-9
     assert r["time_to_first_frame_s"]["p99"] <= r["time_to_last_frame_s"]["p50"]
+
+
+def test_bf16_decoder_800_sessions_against_the_oracle_and_a_small_handle(sd):
+    """800 sessions in one pass with ragged encoder lengths up to 128: ff1 and (in start) xkv run on 128 x 256 tiles and k_attend on up to
+    128 encoder positions.  Seven sessions (rows 0, 127, 128, 767, 768, 799 and the longest encoder sequence) are each >= 40 dB from the
+    oracle run for that session alone, and bitwise what a handle of seven sessions (128 x 128 and 64-wide tiles throughout) gives them."""
+    from infernos_b200.engine import TTSDecoder
+    n, L = 800, 128
+    g = torch.Generator().manual_seed(51)
+    lens = torch.randint(1, L + 1, (n,), generator=g, dtype=torch.int32)
+    lens[400], lens[401] = 1, L
+    enc, spk = synth.synth_encoder_states(n, L, seed=52), synth.synth_speakers(n, seed=53)
+    masks = (torch.rand(16, 2, 256, generator=g) < 0.5).float()
+    pick = sorted({0, 127, 128, 767, 768, 799, int(lens.argmax())})
+    big = TTSDecoder("cuda:0", sd, mode="bf16", max_sessions=n, max_steps=32, max_enc_len=L)
+    try:
+        slots = torch.arange(n, dtype=torch.int32).cuda()
+        big.start(slots, enc.cuda(), lens.cuda(), spk.cuda())
+        mel, _ = big.steps(slots, 16, masks=masks.cuda())
+        big.poll_errors()
+        mel = mel.cpu()
+    finally:
+        big.close()
+    small = TTSDecoder("cuda:0", sd, mode="bf16", max_sessions=len(pick), max_steps=32, max_enc_len=L)
+    try:
+        ps = torch.arange(len(pick), dtype=torch.int32).cuda()
+        small.start(ps, enc[pick].cuda(), lens[pick].cuda(), spk[pick].cuda())
+        mel_small, _ = small.steps(ps, 16, masks=masks.cuda())
+        small.poll_errors()
+        mel_small = mel_small.cpu()
+    finally:
+        small.close()
+    for j, i in enumerate(pick):
+        n_i = int(lens[i])
+        ref, _ = _oracle(sd, enc[i:i + 1, :n_i], torch.ones(1, n_i, dtype=torch.int), spk[i:i + 1], masks)
+        c = ref.mean()
+        snr = _snr(ref[0] - c, mel[i] - c)
+        same = torch.equal(mel[i], mel_small[j])
+        print(f"decoder bf16, 800 sessions: session {i} ({n_i} encoder positions) SNR {snr:.2f} dB, bitwise equal on a 7-session handle: {same}")
+        assert snr >= 40.0, (i, snr)
+        assert same, f"session {i}: an 800-session pass does not give the bits a 7-session handle gives"
+
+
+def test_fp32_decoder_128_steps_over_long_encoder_sequences(sd):
+    """Eight 16-step calls (128 self-attention positions, the KV cache carried across calls) over encoder sequences of 65, 128 and 200
+    positions, against the oracle run over the same 128 steps."""
+    from infernos_b200.engine import TTSDecoder
+    lens, L = [65, 128, 200], 200
+    g = torch.Generator().manual_seed(61)
+    enc, spk = synth.synth_encoder_states(3, L, seed=62), synth.synth_speakers(3, seed=63)
+    mask = (torch.arange(L)[None] < torch.tensor(lens)[:, None]).to(torch.int)
+    masks = (torch.rand(128, 2, 256, generator=g) < 0.5).float()
+    dec = TTSDecoder("cuda:0", sd, mode="fp32", max_sessions=4, max_steps=128, max_enc_len=L)
+    try:
+        slots = torch.tensor([2, 0, 3], dtype=torch.int32).cuda()
+        dec.start(slots, enc.cuda(), torch.tensor(lens, dtype=torch.int32).cuda(), spk.cuda())
+        got = torch.cat([dec.steps(slots, 16, masks=masks[16 * c:16 * c + 16].cuda())[0].cpu() for c in range(8)], 1)
+        dec.poll_errors()
+        assert [dec.get_step(s) for s in (2, 0, 3)] == [128] * 3
+    finally:
+        dec.close()
+    ref, _ = _oracle(sd, enc, mask, spk, masks)
+    ref64, _ = _oracle({k: v.double() for k, v in sd.items()}, enc.double(), mask, spk.double(), masks.double())
+    per_call = [float((got[:, 32 * c:32 * c + 32] - ref[:, 32 * c:32 * c + 32]).abs().max()) for c in range(8)]
+    drift = float((ref.double() - ref64).abs().max())
+    print(f"decoder fp32, 128 steps, encoder lengths {lens}: max |d mel| per 16-step call {', '.join(f'{e:.1e}' for e in per_call)}; "
+          f"against the float64 oracle {float((got.double() - ref64).abs().max()):.1e}; the oracle's own float32-vs-float64 drift {drift:.1e}")
+    assert max(per_call) <= 1e-3

@@ -239,3 +239,70 @@ def test_bf16_encoder_into_the_bf16_decoder_against_the_oracle_encoder_states():
     snr = _snr(mel[3:] - c, mel[:3] - c)
     print(f"bf16 GPU encoder -> bf16 decoder vs oracle encoder states -> same decoder: mel SNR {snr:.2f} dB")
     assert snr >= 40.0
+
+
+def _sms():
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def test_bf16_encoder_one_large_pass_is_bitwise_each_sentence_alone(sd):
+    """About 4,000 rows in one pass of the default 16,384-row workspace: there qkv and ff1 run on 128 x 256 tiles, while each sentence alone
+    (at most 200 rows) runs them on 128 x 128 tiles.  Every sentence's rows must still be bitwise what it gets alone on the same handle, padded
+    rows zero, and six of them (the first, the last, the longest and three more) within the usual floors of the oracle."""
+    from infernos_b200.engine import TTSEncoder
+    g = torch.Generator().manual_seed(41)
+    lengths = [int(x) for x in torch.randint(8, 201, (40,), generator=g)]
+    ids, mask = synth.synth_token_ids(lengths, seed=42)
+    rows = sum(lengths)
+    assert -(-rows // 128) * (2304 // 128) > _sms(), f"{rows} rows do not put qkv (N = 2304) on 128 x 256 tiles"
+    enc = TTSEncoder("cuda:0", sd, mode="bf16")
+    try:
+        cohort = enc(ids, mask).cpu()
+        alone = [enc(ids[i:i + 1, :n], None).cpu()[0] for i, n in enumerate(lengths)]
+        enc.poll_errors()
+    finally:
+        enc.close()
+    m = mask.bool()
+    assert float(cohort[~m].abs().max()) == 0.0, "padded rows must be zero"
+    diff = [i for i, n in enumerate(lengths) if not torch.equal(cohort[i, :n], alone[i])]
+    print(f"encoder bf16, {len(lengths)} sentences, {rows} rows in one pass: {len(lengths) - len(diff)} of {len(lengths)} bitwise equal to alone")
+    assert not diff, f"sentences {diff}: a {rows}-row pass does not give the bits they get alone"
+    longest = max(range(len(lengths)), key=lambda i: lengths[i])
+    pick = sorted({0, len(lengths) - 1, longest, 10, 20, 30})
+    Lp = max(lengths[i] for i in pick)
+    sub_ids, sub_mask = ids[pick, :Lp], mask[pick, :Lp]
+    _check("bf16", _oracle(sd, sub_ids, sub_mask)[sub_mask.bool()], cohort[pick, :Lp], sub_mask, f"sentences {pick} of a {rows}-row pass")
+
+
+@pytest.mark.parametrize("max_tokens,lengths", [(64, (64, 30, 9, 57, 1)), (100, (100, 37, 63, 1, 88))])
+def test_bf16_encoder_workspace_smaller_than_one_tile(sd, max_tokens, lengths):
+    """max_tokens below the GEMM's 128-row box: the A maps span fewer rows than one tile, every pass is cut short of it.  Against the oracle,
+    and bitwise against a handle with the default workspace."""
+    from infernos_b200.engine import TTSEncoder
+    ids, mask = synth.synth_token_ids(lengths, seed=44 + max_tokens)
+    small = TTSEncoder("cuda:0", sd, mode="bf16", max_tokens=max_tokens, max_len=128)
+    big = TTSEncoder("cuda:0", sd, mode="bf16", max_len=128)
+    try:
+        got = small(ids, mask).cpu()
+        ref_big = big(ids, mask).cpu()
+        small.poll_errors(); big.poll_errors()
+    finally:
+        small.close(); big.close()
+    _check("bf16", _oracle(sd, ids, mask)[mask.bool()], got, mask, f"max_tokens {max_tokens}")
+    assert torch.equal(got, ref_big)
+
+
+def test_fp32_encoder_lengths_at_the_attention_tile_edges(sd):
+    """k_enc_attend works on key tiles of 32 and query tiles of 64; lengths on either side of their edges, and the whole positional table
+    (450).  The oracle runs per sentence at its own length."""
+    from infernos_b200.engine import TTSEncoder
+    lengths = (31, 32, 33, 63, 64, 65, 127, 128, 129, 320, 450)
+    ids, mask = synth.synth_token_ids(lengths, seed=43)
+    enc = TTSEncoder("cuda:0", sd, mode="fp32", max_tokens=2048, max_len=450)
+    try:
+        got = enc(ids, mask).cpu()
+        enc.poll_errors()
+    finally:
+        enc.close()
+    ref = torch.cat([_oracle(sd, ids[i:i + 1, :n], None)[0] for i, n in enumerate(lengths)])
+    _check("fp32", ref, got, mask, "lengths at the attention kernel's tile edges")
