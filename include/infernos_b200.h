@@ -274,7 +274,7 @@ B2_API int b2_resblock_tc(const float *d_x, const float *h_weights, const float 
  * out[10] = {S rows per slab, H halo, V output rows per tile, tiles per window, off[0..2], lim[0..2]}: conv1 of pair i reads slab rows
  * [off[i], off[i] + lim[i]) through the operand mapping of dilation d_i.  Returns non-zero (b2_last_error) when the kernel does not cover the shape. */
 B2_API int b2_resblock_t_plan(int k, int d0, int d1, int d2, int T, int post, int *out);
-/* Test hook: C = 32 ResBlocks with at least k taps run the stacked-output kernel (default 5, B2_RB_T_MINK; measured: three-tap blocks are
+/* Test hook: C = 32 ResBlocks with at least k taps run the stacked-output kernel (default 5; measured: three-tap blocks are
  * faster on the time-as-M kernel).  k <= 0 restores the default.  Process-wide; not for concurrent use with running launches. */
 B2_API int b2_debug_set_stacked_min_taps(int k);
 

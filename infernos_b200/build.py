@@ -30,7 +30,7 @@ def needs_build() -> bool:
 
 
 def build(force: bool = False, verbose: bool = False, extra_flags=(), so_out: str = SO, tag: str = "") -> str:
-    """extra_flags / out / tag: variant builds for A/B runs (e.g. -DB2_MBAR_NO_HINT into libinfernos_b200_nohint.so; load with B2_SO_PATH)."""
+    """extra_flags / out / tag: variant builds (e.g. -DB2_RBT_ZERO_INIT into libinfernos_b200_zeroinit.so; load with B2_SO_PATH)."""
     if not force and not extra_flags and not needs_build():
         return SO
     objs = []
@@ -55,7 +55,7 @@ def build(force: bool = False, verbose: bool = False, extra_flags=(), so_out: st
 
 
 if __name__ == "__main__":
-    if "--variant" in sys.argv:          # python -m infernos_b200.build --variant nohint -DB2_MBAR_NO_HINT
+    if "--variant" in sys.argv:          # python -m infernos_b200.build --variant zeroinit -DB2_RBT_ZERO_INIT
         i = sys.argv.index("--variant")
         name, flags = sys.argv[i + 1], [a for a in sys.argv[i + 2:] if a.startswith("-D")]
         print(build(force=True, extra_flags=flags, so_out=os.path.join(HERE, f"libinfernos_b200_{name}.so"), tag="_" + name))

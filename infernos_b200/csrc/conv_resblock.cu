@@ -62,9 +62,6 @@ struct RbParams {
     int dil0, dil1, dil2;
     unsigned long long m_tpw;
     unsigned long long *dbg;   // optional per-CTA phase timestamps (B2_RB_DBG analysis runs)
-    int dbg_flags;             // bit 0: no L2 prefetch of the slab at CTA start (B2_RB_NOPF=1: A/B switch); bit 1: what-if, timing only (B2_RB_NORING=1): no weight
-                               // ring at all -- no TMA loads, no full / empty barrier traffic, the MMAs read whatever the ring area holds
-    int pf_dist;               // > 0: also prefetch the slab of CTA blockIdx.x + pf_dist into L2 (the CTA that follows this one on the SM)
     float bias1[3 * kRbMaxC];  // conv1 biases                                         (constant bank: uniform loads)
     float cbias[3 * kRbMaxC];  // running sum of conv2 biases: cbias[i] = b2[0] + .. + b2[i]
 };
@@ -79,27 +76,6 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32
           "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]),
           "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
         : "memory");
-}
-
-// two 32-column TMEM loads in flight, one wait (the pair epilogue: their latencies overlap)
-__device__ __forceinline__ void tmem_ld32x2(uint32_t ta, uint32_t tb, uint32_t (&a)[32], uint32_t (&b)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%64];\n\t"
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%32, %33, %34, %35, %36, %37, %38, %39, %40, %41, %42, %43, %44, %45, %46, %47, "
-        "%48, %49, %50, %51, %52, %53, %54, %55, %56, %57, %58, %59, %60, %61, %62, %63}, [%65];\n\t"
-        "tcgen05.wait::ld.sync.aligned;"
-        : "=r"(a[0]), "=r"(a[1]), "=r"(a[2]), "=r"(a[3]), "=r"(a[4]), "=r"(a[5]), "=r"(a[6]), "=r"(a[7]),
-          "=r"(a[8]), "=r"(a[9]), "=r"(a[10]), "=r"(a[11]), "=r"(a[12]), "=r"(a[13]), "=r"(a[14]), "=r"(a[15]),
-          "=r"(a[16]), "=r"(a[17]), "=r"(a[18]), "=r"(a[19]), "=r"(a[20]), "=r"(a[21]), "=r"(a[22]), "=r"(a[23]),
-          "=r"(a[24]), "=r"(a[25]), "=r"(a[26]), "=r"(a[27]), "=r"(a[28]), "=r"(a[29]), "=r"(a[30]), "=r"(a[31]),
-          "=r"(b[0]), "=r"(b[1]), "=r"(b[2]), "=r"(b[3]), "=r"(b[4]), "=r"(b[5]), "=r"(b[6]), "=r"(b[7]),
-          "=r"(b[8]), "=r"(b[9]), "=r"(b[10]), "=r"(b[11]), "=r"(b[12]), "=r"(b[13]), "=r"(b[14]), "=r"(b[15]),
-          "=r"(b[16]), "=r"(b[17]), "=r"(b[18]), "=r"(b[19]), "=r"(b[20]), "=r"(b[21]), "=r"(b[22]), "=r"(b[23]),
-          "=r"(b[24]), "=r"(b[25]), "=r"(b[26]), "=r"(b[27]), "=r"(b[28]), "=r"(b[29]), "=r"(b[30]), "=r"(b[31])
-        : "r"(ta), "r"(tb));
 }
 
 // 32 consecutive fp32 of one row (128 bytes) -> registers; zeros when the row is not wanted
@@ -136,12 +112,6 @@ __device__ __forceinline__ void write_operand_row(uint32_t sA_u32, int r, int c0
 #pragma unroll
         for (int e = 0; e < 4; e++) {
             const int c = 8 * i + 2 * e;
-#ifdef B2_RB_SCALAR_EPI          // the round-1 scalar form (variant build for A/B runs; same results)
-            float v0 = __uint_as_float(v[c]), v1 = __uint_as_float(v[c + 1]);
-            if (bias) { v0 += bias[c]; v1 += bias[c + 1]; }
-            const float m0 = v0 * slope, m1 = v1 * slope;
-            (void)slope2;
-#else
             unsigned long long x2 = rb_pack2(__uint_as_float(v[c]), __uint_as_float(v[c + 1]));
             if (bias) asm("add.rn.f32x2 %0, %1, %2;" : "=l"(x2) : "l"(x2), "l"(rb_pack2(bias[c], bias[c + 1])));
             unsigned long long m2;
@@ -149,7 +119,6 @@ __device__ __forceinline__ void write_operand_row(uint32_t sA_u32, int r, int c0
             float v0, v1, m0, m1;
             asm("mov.b64 {%0, %1}, %2;" : "=f"(v0), "=f"(v1) : "l"(x2));
             asm("mov.b64 {%0, %1}, %2;" : "=f"(m0), "=f"(m1) : "l"(m2));
-#endif
             __nv_bfloat162 h2 = __floats2bfloat162_rn(fmaxf(v0, m0), fmaxf(v1, m1));
             pk[e] = *reinterpret_cast<uint32_t *>(&h2);
         }
@@ -170,14 +139,6 @@ __device__ __forceinline__ void publish_rows(uint32_t bar, int lane) {
     if (lane == 0) mbar_arrive(bar);
 }
 
-// the same for two sub-tiles at once: one pair of fences, two arrivals
-__device__ __forceinline__ void publish_rows2(uint32_t bar_a, uint32_t bar_b, int lane) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncwarp();
-    if (lane == 0) { mbar_arrive(bar_a); mbar_arrive(bar_b); }
-}
-
 static constexpr int kRbDbgEvents = 48, kRbDbgCtas = 4096;
 #define RB_DBG(k) do { if (DBG && p.dbg && blockIdx.x < kRbDbgCtas) p.dbg[(size_t)blockIdx.x * kRbDbgEvents + (k)] = clock64(); } while (0)
 
@@ -187,15 +148,8 @@ static constexpr int kRbDbgEvents = 48, kRbDbgCtas = 4096;
 // EPI selects the final epilogue at compile time (its code is a third of the kernel, and the kernel has to fit the instruction
 // cache): 0 out32 = r;  1 out32 = acc + r;  2 outb = bf16(lrelu((acc + r) / div));  3 out32 = (acc + r) / div;  4 everything decided at run time;
 // 5 (C = 32 only) the vocoder's last step fused in: audio = tanh(conv_post(lrelu((acc + r) / div, 0.01))), nothing else written.
-// C = 32 with NEW = 8 ("sub-tile split"): two CTAs still share an SM, and warps 4..7 take the ODD sub-tiles of every phase (slab load,
-// the six conv epilogues, the final epilogue) that warps 0..3 used to do alone: the epilogue chain of a conv, which bounded the C = 32
-// launches (profiles/r1d_resblock_phase_timestamps.txt: ~3k cycles per conv for ~1k cycles of MMA issue), is walked by twice the warps.
-// PAIR: the conv epilogues take the sub-tiles two at a time -- both TMEM loads in flight before either is consumed, one proxy fence and one
-// barrier hand-shake per pair instead of per sub-tile.  At C = 32 / 64 with short filters the epilogue warps are the busiest resource of
-// the CTA (each conv costs them kS x ~750 cycles, mostly latency: TMEM load, proxy fence, barrier round trip), so this is where a cycle saved
-// is a cycle off the step.
-template <int C, int NEW, int NMW, int EPI, bool DBG, bool PAIR>
-__global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? (NEW == 8 ? 88 : 128) : 168) k_resblock(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ RbParams p) {
+template <int C, int NEW, int NMW, int EPI, bool DBG>
+__global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 128 : 168) k_resblock(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ RbParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     pdl_trigger();
     using G = RbGeom<C>;
@@ -203,16 +157,13 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     constexpr int kThreads = (NEW + 1 + NMW) * 32;
     constexpr int CH = C / 32;                                  // 32-column chunks per row
-    constexpr bool SSPLIT = (C == 32 && NEW == 8);              // epilogue warps 4..7 own the odd sub-tiles instead of a column slice
-    constexpr int SSTEP = SSPLIT ? 2 : 1;
-    constexpr int CHW = SSPLIT ? CH : CH / (NEW / 4);           // ... of which one epilogue warp handles CHW
-    constexpr int NCHW = (kS / SSTEP) * CHW;                    // 32x32 pieces per epilogue warp
-    constexpr int READY_CNT = SSPLIT ? 4 : NEW;                 // warps that publish one sub-tile
-    constexpr uint32_t kStgBytes = SSPLIT ? 4096u : 8192u;      // per-warp staging of the slab load (A2 holds NEW of them)
+    constexpr int CHW = CH / (NEW / 4);                         // ... of which one epilogue warp handles CHW
+    constexpr int NCHW = kS * CHW;                              // 32x32 pieces per epilogue warp
+    constexpr uint32_t kStgBytes = 8192u;                       // per-warp staging of the slab load (A2 holds NEW of them)
     constexpr int SPW = kS / NMW;                               // sub-tiles per MMA warp
     constexpr uint32_t kTapKbBytes = (uint32_t)C * KB * 2;      // one tap, one K block
     constexpr uint32_t kABytes = G::kABytes;
-    static_assert((SSPLIT || CH % (NEW / 4) == 0) && kS % NMW == 0 && 2 * kS * C <= 512 && NEW * kStgBytes <= G::kABytes, "unsupported geometry");
+    static_assert(CH % (NEW / 4) == 0 && kS % NMW == 0 && 2 * kS * C <= 512 && NEW * kStgBytes <= G::kABytes, "unsupported geometry");
     const uint32_t slot_bytes = (uint32_t)p.tps * kTapKbBytes;
     uint8_t *sW = smem;
     uint8_t *sA1 = smem + (size_t)p.nslots * slot_bytes;
@@ -236,34 +187,13 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
     // The slab's x rows (and, for the final epilogue, the MRF partial sum's) start their way from HBM into L2 before anything else:
     // the load phase below keeps only two 4 KB pieces per warp in flight, so at HBM latency it was ~13k cycles of a 34-114k-cycle CTA
     // (phase timestamps, profiles/); out of L2 it is a few thousand.  One 128-byte line per lane per 32-channel piece.
-    if (warp < NEW && !(p.dbg_flags & 1)) {
-        const int rq0 = (warp & 3) * 32 + lane, cb0 = SSPLIT ? 0 : (warp >> 2) * (CHW * 32);
+    if (warp < NEW) {
+        const int rq0 = (warp & 3) * 32 + lane, cb0 = (warp >> 2) * (CHW * 32);
 #pragma unroll
-        for (int s = SSPLIT ? (warp >> 2) : 0; s < kS; s += SSTEP) {
+        for (int s = 0; s < kS; s++) {
             const int r = s * 128 + rq0, t = t_base + r;
             if (t >= 0 && t < p.T) {
                 const size_t off = ((size_t)w * p.T + t) * C + cb0;
-#pragma unroll
-                for (int cc = 0; cc < CHW; cc++) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.x + off + cc * 32));
-                if (p.acc_src && r >= p.H && r < p.H + p.V) {
-#pragma unroll
-                    for (int cc = 0; cc < CHW; cc++) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.acc_src + off + cc * 32));
-                }
-            }
-        }
-    }
-    // ... and the slab of the CTA that will take this one's place on the SM (pf_dist CTAs ahead: one resident set) is requested NOW, a whole
-    // CTA lifetime before it is needed, so that its own load phase finds the rows in L2 instead of waiting ~2 us for HBM.
-    if (warp < NEW && p.pf_dist > 0 && blockIdx.x + (unsigned)p.pf_dist < gridDim.x) {
-        const int b2i = (int)blockIdx.x + p.pf_dist;
-        const int w2 = fdiv(b2i, p.m_tpw);
-        const int tb2 = (b2i - w2 * p.tiles_per_win) * p.V - p.H;
-        const int rq0 = (warp & 3) * 32 + lane, cb0 = SSPLIT ? 0 : (warp >> 2) * (CHW * 32);
-#pragma unroll
-        for (int s = SSPLIT ? (warp >> 2) : 0; s < kS; s += SSTEP) {
-            const int r = s * 128 + rq0, t = tb2 + r;
-            if (t >= 0 && t < p.T) {
-                const size_t off = ((size_t)w2 * p.T + t) * C + cb0;
 #pragma unroll
                 for (int cc = 0; cc < CHW; cc++) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.x + off + cc * 32));
                 if (p.acc_src && r >= p.H && r < p.H + p.V) {
@@ -279,7 +209,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
             if (smem_u32(smem) & 1023u) __trap();
             asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap_w) : "memory");
             for (int s = 0; s < 4; s++) { mbar_init(W_FULL(s), 1); mbar_init(W_EMPTY(s), NMW); }
-            for (int s = 0; s < kS; s++) { mbar_init(A1_READY(s), READY_CNT); mbar_init(T1_FULL(s), 1); mbar_init(A2_READY(s), READY_CNT); mbar_init(X_FULL(s), 1); }
+            for (int s = 0; s < kS; s++) { mbar_init(A1_READY(s), NEW); mbar_init(T1_FULL(s), 1); mbar_init(A2_READY(s), NEW); mbar_init(X_FULL(s), 1); }
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         }
         __syncwarp();
@@ -312,8 +242,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
     if (warp < NEW) {
         // ======================================================================================= slab load + epilogues
         const int quad = warp & 3;                             // TMEM lane quadrant this warp may touch
-        const int cbase = SSPLIT ? 0 : (warp >> 2) * (CHW * 32);   // first column of this warp's slice
-        const int s0 = SSPLIT ? (warp >> 2) : 0;               // first sub-tile this warp owns (then every SSTEP-th)
+        const int cbase = (warp >> 2) * (CHW * 32);            // first column of this warp's slice
         const int rq = quad * 32 + lane;                       // row inside a sub-tile == TMEM lane
         const uint32_t tm_lane = (uint32_t)(quad * 32) << 16;
         const uint32_t a1_u32 = smem_u32(sA1), a2_u32 = smem_u32(sA2);
@@ -340,8 +269,8 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
             const uint32_t stg_u32 = a2_u32 + (uint32_t)warp * kStgBytes;
             const float *xq = p.x + ((size_t)w * p.T + (t_base + quad * 32 + sub_r)) * C + cbase + c4 * 4;   // row sub_r of this warp's rows in sub-tile 0
             auto issue_piece = [&](int q) {
-                const int s1 = s0 + (q / CHW) * SSTEP, c1 = (q % CHW) * 32;
-                const uint32_t dst0 = stg_u32 + (SSPLIT ? 0u : (uint32_t)((q & 1) * 4096));
+                const int s1 = q / CHW, c1 = (q % CHW) * 32;
+                const uint32_t dst0 = stg_u32 + (uint32_t)((q & 1) * 4096);
 #pragma unroll
                 for (int j = 0; j < 8; j++) {
                     const int row = j * 4 + sub_r;
@@ -354,8 +283,8 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
             issue_piece(0);
 #pragma unroll 1
             for (int q = 0; q < NCHW; q++) {
-                const int s = s0 + (q / CHW) * SSTEP, c0 = cbase + (q % CHW) * 32;
-                if (!SSPLIT && q + 1 < NCHW) {
+                const int s = q / CHW, c0 = cbase + (q % CHW) * 32;
+                if (q + 1 < NCHW) {
                     issue_piece(q + 1);
                     asm volatile("cp.async.wait_group 1;" ::: "memory");
                 } else {
@@ -364,14 +293,13 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                 __syncwarp();
                 uint32_t v[32];
                 {
-                    const uint32_t src0 = stg_u32 + (SSPLIT ? 0u : (uint32_t)((q & 1) * 4096)) + (uint32_t)(lane * 128);
+                    const uint32_t src0 = stg_u32 + (uint32_t)((q & 1) * 4096) + (uint32_t)(lane * 128);
 #pragma unroll
                     for (int j = 0; j < 8; j++)
                         asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v[4 * j]), "=r"(v[4 * j + 1]), "=r"(v[4 * j + 2]), "=r"(v[4 * j + 3])
                                      : "r"(src0 + (uint32_t)((j ^ (lane & 7)) << 4)) : "memory");
                 }
-                __syncwarp();                  // the buffer is refilled two pieces later (SSPLIT: one buffer per warp, refilled right away --
-                if (SSPLIT && q + 1 < NCHW) issue_piece(q + 1);      // its contents are in registers by now)
+                __syncwarp();                  // the buffer is refilled two pieces later
                 tmem_st32(tmem_X + tm_lane + (uint32_t)(s * C + c0), v);
                 write_operand_row<kRtot>(a1_u32, s * 128 + rq, c0, v, nullptr, p.slope, true);
                 if ((q % CHW) == CHW - 1) {
@@ -409,25 +337,8 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                 const uint32_t dst = e ? a1_u32 : a2_u32;
                 const float *bias = (e ? p.cbias : p.bias1) + i * C + cbase;
                 const uint32_t full0 = e ? X_FULL(0) : T1_FULL(0), ready0 = e ? A1_READY(0) : A2_READY(0);
-                if constexpr (PAIR && !SSPLIT) {
 #pragma unroll 1
-                    for (int s = 0; s < kS; s += 2) {
-                        mbar_wait(full0 + 8u * (uint32_t)s, par);
-                        mbar_wait(full0 + 8u * (uint32_t)(s + 1), par);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        if (threadIdx.x == 0 && s == 0) RB_DBG(3 + 4 * i + 2 * e);
-#pragma unroll 1
-                        for (int cc = 0; cc < CHW; cc++) {
-                            uint32_t acc0[32], acc1[32];
-                            tmem_ld32x2(src + (uint32_t)(s * C + cbase + cc * 32), src + (uint32_t)((s + 1) * C + cbase + cc * 32), acc0, acc1);
-                            write_operand_row<kRtot>(dst, s * 128 + rq, cbase + cc * 32, acc0, bias + cc * 32, p.slope, inside(s));
-                            write_operand_row<kRtot>(dst, (s + 1) * 128 + rq, cbase + cc * 32, acc1, bias + cc * 32, p.slope, inside(s + 1));
-                        }
-                        publish_rows2(ready0 + 8u * (uint32_t)s, ready0 + 8u * (uint32_t)(s + 1), lane);
-                    }
-                } else {
-#pragma unroll 1
-                for (int s = s0; s < kS; s += SSTEP) {
+                for (int s = 0; s < kS; s++) {
                     const bool probe = DBG && threadIdx.x == 0 && i == 1 && e == 0 && s == 1;     // micro-phases of ONE sub-tile's epilogue (analysis build)
                     if (probe) RB_DBG(15);
                     mbar_wait(full0 + 8u * (uint32_t)s, par);
@@ -439,11 +350,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                         uint32_t acc[32];
                         tmem_ld32(src + (uint32_t)(s * C + cbase + cc * 32), acc);
                         if (probe && cc == 0) RB_DBG(30);
-#ifdef B2_RB_EXP_NOBIAS          // timing experiment only (wrong results): what the conv epilogue costs without the bias add
-                        write_operand_row<kRtot>(dst, s * 128 + rq, cbase + cc * 32, acc, nullptr, p.slope, inside(s));
-#else
                         write_operand_row<kRtot>(dst, s * 128 + rq, cbase + cc * 32, acc, bias + cc * 32, p.slope, inside(s));
-#endif
                     }
                     if (probe) RB_DBG(31);
                     if constexpr (DBG) {
@@ -456,7 +363,6 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                     } else {
                         publish_rows(ready0 + 8u * (uint32_t)s, lane);
                     }
-                }
                 }
                 if (threadIdx.x == 0) RB_DBG(4 + 4 * i + 2 * e);
             }
@@ -476,7 +382,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                     for (int q = threadIdx.x; q < 7 * 32; q += NEW * 32) wp[q] = __ldg(p.post_w + q);
                     // pass A (lane owns a row): X + running bias -> V
 #pragma unroll 1
-                    for (int s = s0; s < kS; s += SSTEP) {
+                    for (int s = 0; s < kS; s++) {
                         uint32_t a32[32];
                         tmem_ld32(tmem_X + tm_lane + (uint32_t)(s * C), a32);
                         const float *cb = p.cbias + 2 * C;
@@ -495,7 +401,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                         const float rcp = p.rdiv, nd = -p.div;
                         const float *aq = p.acc_src + ((size_t)w * p.T + (t_base + quad * 32 + sub_r)) * C + c4 * 4;
 #pragma unroll 1
-                        for (int s = s0; s < kS; s += SSTEP) {
+                        for (int s = 0; s < kS; s++) {
                             float4 acc4[8];
 #pragma unroll
                             for (int j = 0; j < 8; j++)
@@ -556,7 +462,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                 const size_t row0 = (size_t)w * p.T + (t_base + quad * 32 + sub_r);        // global row of (sub-tile 0, j = 0)
                 const float *aq = p.acc_src + row0 * C + cbase + c4 * 4;            // only dereferenced when the epilogue has an acc_src
                 auto ld_acc = [&](int q, float4 (&b)[8]) {
-                    const int s1 = s0 + (q / CHW) * SSTEP, c1 = (q % CHW) * 32;
+                    const int s1 = q / CHW, c1 = (q % CHW) * 32;
 #pragma unroll
                     for (int j = 0; j < 8; j++)
                         b[j] = ((out_t[j] >> s1) & 1u) ? *reinterpret_cast<const float4 *>(aq + ((size_t)s1 * 128 + j * 4) * C + c1) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -565,11 +471,9 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                 const bool has_div = (EPI == 4) ? (p.div != 1.0f) : (EPI >= 2);
                 const bool has_o32 = (EPI == 4) ? (p.out32 != nullptr) : (EPI != 2);
                 const bool has_ob = (EPI == 4) ? (p.outb != nullptr) : (EPI == 2);
-                // register prefetch of the NEXT piece's partial sums; not with eight epilogue warps at C = 32 (88 registers per thread:
-                // the second buffer would spill), where the loads of the current piece are issued ahead of its TMEM read instead
-                constexpr bool PF = !SSPLIT;
+                // register prefetch of the NEXT piece's partial sums
                 float4 accA[8], accB[8];
-                if (has_acc && PF) ld_acc(0, accA);
+                if (has_acc) ld_acc(0, accA);
                 if (threadIdx.x == 0) RB_DBG(40);
                 const float rcp = p.rdiv, nd = -p.div;
                 // One 32x32 piece.  `cur` holds its partial sums; the next piece's are requested into `nxt` while this one is worked on, and the two
@@ -578,14 +482,13 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                 // store; }` the compiler emitted a divergent branch and a load -> store round trip per row, one after the other (round 2: ~1.4k
                 // cycles per piece in the stacked-output kernel, whose final epilogue had the same shape).
                 auto piece = [&](int q, float4 (&cur)[8], float4 (&nxt)[8]) {
-                    const int s = s0 + (q / CHW) * SSTEP, c0 = cbase + (q % CHW) * 32;
+                    const int s = q / CHW, c0 = cbase + (q % CHW) * 32;
                     if ((q % CHW) == 0) {
                         mbar_wait(X_FULL(s), par);
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                         if (threadIdx.x == 0 && s == 0) RB_DBG(5 + 4 * i);
                         if (threadIdx.x == 0) RB_DBG(32 + s);
                     }
-                    if (has_acc && !PF) ld_acc(q, cur);
                     {
                         uint32_t a32[32];
                         tmem_ld32(tmem_X + tm_lane + (uint32_t)(s * C + c0), a32);
@@ -597,7 +500,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                             *reinterpret_cast<uint4 *>(stg + lane * kRbStageLd + j * 4) = make_uint4(a32[4 * j], a32[4 * j + 1], a32[4 * j + 2], a32[4 * j + 3]);
                     }
                     __syncwarp();
-                    if (has_acc && PF && q + 1 < NCHW) ld_acc(q + 1, nxt);
+                    if (has_acc && q + 1 < NCHW) ld_acc(q + 1, nxt);
 #pragma unroll
                     for (int jh = 0; jh < 8; jh += 4) {
                         float4 v[4];
@@ -649,7 +552,6 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
             for (int c = 0; c < 6; c++)
                 for (int g = 0; g < p.ngroups; g++)
                     for (int kb = 0; kb < NKB; kb++) {
-                        if (p.dbg_flags & 2) continue;
                         mbar_wait(W_EMPTY(slot), phase ^ 1);
                         mbar_expect_tx(W_FULL(slot), slot_bytes);
                         tma_load_3d(smem_u32(sW + (size_t)slot * slot_bytes), &tmap_w, W_FULL(slot), kb * KB, 0, c * p.taps + g * p.tps);
@@ -692,7 +594,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                         const int ntap = min(p.tps, p.taps - j0);
 #pragma unroll 1
                         for (int kb = 0; kb < NKB; kb++) {
-                            if (!(p.dbg_flags & 2)) mbar_wait(W_FULL(slot), phase);
+                            mbar_wait(W_FULL(slot), phase);
                             const uint64_t bdesc_g = bdesc0 + (uint64_t)((uint32_t)slot * slot_16);
                             const bool first = (g == 0) && (kb == 0), last = (g == p.ngroups - 1) && (kb == NKB - 1);
 #pragma unroll 1
@@ -722,7 +624,7 @@ __global__ void __launch_bounds__((NEW + 1 + NMW) * 32) __maxnreg__((C == 32) ? 
                                 }
                                 if (last) umma_commit(done0 + 8u * (uint32_t)s);
                             }
-                            if (!(p.dbg_flags & 2)) umma_commit(W_EMPTY(slot));
+                            umma_commit(W_EMPTY(slot));
                             if (++slot == p.nslots) { slot = 0; phase ^= 1; }
                         }
                     }
@@ -823,56 +725,36 @@ void resblock_free(ResBlockPack &p) {
 }
 
 
-static bool g_rb_attr[64][4][14] = {};
+static bool g_rb_attr[64][3][7] = {};
 
-template <int C, int NEW, int NMW, int EPI, bool DBG, bool PAIR>
-static int launch_rb__(const CUtensorMap &tm, const RbParams &p, unsigned grid, size_t smem, cudaStream_t st, int wslot) {
-    int dev = 0;
-    B2_CUDA_OK(cudaGetDevice(&dev));
-    const int eslot = (DBG ? 6 : EPI) + (PAIR ? 7 : 0);
-    if (dev < 64 && !g_rb_attr[dev][wslot][eslot]) {
-        B2_CUDA_OK(cudaFuncSetAttribute(k_resblock<C, NEW, NMW, EPI, DBG, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        g_rb_attr[dev][wslot][eslot] = true;
-    }
-    B2_CUDA_OK(launch_k(k_resblock<C, NEW, NMW, EPI, DBG, PAIR>, dim3(grid), dim3((NEW + 1 + NMW) * 32), smem, st, pdl_enabled(), tm, p));
-    B2_LAUNCH_OK("k_resblock");
-    return 0;
-}
-
-// B2_RB_PAIR=1 runs the paired conv epilogue.  Measured on the B200 (profiles/r2i_ab_paired_epilogue.json): bit-identical results, but no
-// faster -- the nine ResBlock launches 15.37 ms paired against 14.77 ms unpaired in the same run: waiting for the second sub-tile's MMAs before
-// touching the first delays the hand-off to the next convolution by more than the shared fence saves.  Off by default.
-template <int C, int NEW, int NMW, int EPI, bool DBG>
-static int launch_rb_(const CUtensorMap &tm, const RbParams &p, unsigned grid, size_t smem, cudaStream_t st, int wslot) {
-    static const bool pair_on = getenv("B2_RB_PAIR") && atoi(getenv("B2_RB_PAIR")) != 0;
-    if constexpr (!DBG && NEW != 8 || C != 32) {
-        if (pair_on && !DBG) return launch_rb__<C, NEW, NMW, EPI, false, true>(tm, p, grid, smem, st, wslot);
-    }
-    return launch_rb__<C, NEW, NMW, EPI, DBG, false>(tm, p, grid, smem, st, wslot);
-}
-
-// picks the compile-time epilogue that matches the request (the vocoder's three launches per stage are EPI 0, 1 and 2 or 3);
-// anything else, and the timestamped analysis build, runs the generic kernel
+// launches the instantiation whose compile-time epilogue matches the request (the vocoder's three launches per stage are EPI 0, 1 and 2
+// or 3); anything else, and the timestamped analysis build, runs the generic kernel
 template <int C, int NEW, int NMW>
 static int launch_rb(const CUtensorMap &tm, const RbParams &p, unsigned grid, size_t smem, cudaStream_t st, int wslot) {
-    if (p.dbg) return launch_rb_<C, NEW, NMW, 4, true>(tm, p, grid, smem, st, wslot);
+    int dev = 0;
+    B2_CUDA_OK(cudaGetDevice(&dev));
+    auto go = [&](void (*kern)(CUtensorMap, RbParams), int eslot) -> int {
+        if (dev < 64 && !g_rb_attr[dev][wslot][eslot]) {
+            B2_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            g_rb_attr[dev][wslot][eslot] = true;
+        }
+        B2_CUDA_OK(launch_k(kern, dim3(grid), dim3((NEW + 1 + NMW) * 32), smem, st, pdl_enabled(), tm, p));
+        B2_LAUNCH_OK("k_resblock");
+        return 0;
+    };
+    if (p.dbg) return go(k_resblock<C, NEW, NMW, 4, true>, 6);
     if constexpr (C == 32) {
-        if (p.audio) return launch_rb_<C, NEW, NMW, 5, false>(tm, p, grid, smem, st, wslot);
+        if (p.audio) return go(k_resblock<C, NEW, NMW, 5, false>, 5);
     }
     const bool acc = p.acc_src != nullptr, dv = p.div != 1.0f, o32 = p.out32 != nullptr, ob = p.outb != nullptr;
-    if (!acc && !dv && o32 && !ob) return launch_rb_<C, NEW, NMW, 0, false>(tm, p, grid, smem, st, wslot);
-    if (acc && !dv && o32 && !ob) return launch_rb_<C, NEW, NMW, 1, false>(tm, p, grid, smem, st, wslot);
-    if (acc && dv && !o32 && ob) return launch_rb_<C, NEW, NMW, 2, false>(tm, p, grid, smem, st, wslot);
-    if (acc && dv && o32 && !ob) return launch_rb_<C, NEW, NMW, 3, false>(tm, p, grid, smem, st, wslot);
-    return launch_rb_<C, NEW, NMW, 4, false>(tm, p, grid, smem, st, wslot);
+    if (!acc && !dv && o32 && !ob) return go(k_resblock<C, NEW, NMW, 0, false>, 0);
+    if (acc && !dv && o32 && !ob) return go(k_resblock<C, NEW, NMW, 1, false>, 1);
+    if (acc && dv && !o32 && ob) return go(k_resblock<C, NEW, NMW, 2, false>, 2);
+    if (acc && dv && o32 && !ob) return go(k_resblock<C, NEW, NMW, 3, false>, 3);
+    return go(k_resblock<C, NEW, NMW, 4, false>, 4);
 }
 
 int g_rbt_min_taps = 0;
-
-bool resblock_t_enabled() {
-    static const bool on = !(getenv("B2_RB_T") && atoi(getenv("B2_RB_T")) == 0);
-    return on;
-}
 
 int launch_resblock(const ResBlockArgs &a, cudaStream_t st) {
     const ResBlockPack &pk = *a.pack;
@@ -885,14 +767,11 @@ int launch_resblock(const ResBlockArgs &a, cudaStream_t st) {
         if (!pk.tmap_t) return set_error("resblock: the fused upsampler needs the stacked-output kernel (C = 32)");
         return launch_resblock_t(a, st);
     }
-    // C = 32, five taps and more: the stacked-output kernel (conv_resblock_t.cu).  B2_RB_T=0 keeps this file's time-as-M kernel for A/B runs and
-    // the variant tests; B2_RB_T_MINK sets the smallest tap count that goes to the stacked kernel.  Measured (ncu, 4,096 windows, same run):
+    // C = 32, five taps and more: the stacked-output kernel (conv_resblock_t.cu).  Measured (ncu, 4,096 windows, same run):
     // k = 11 2.73 vs 3.57 ms, k = 7 1.85 vs 2.01 ms, but k = 3 1.44 vs 1.34 ms -- with three taps half of the stacked MMAs' N range is
     // structural zeros and the conv epilogues, not the MMAs, set the pace in both kernels.
-    const bool rbt_on = resblock_t_enabled();
-    static const int rbt_mink_env = getenv("B2_RB_T_MINK") ? atoi(getenv("B2_RB_T_MINK")) : 5;
-    const int rbt_mink = g_rbt_min_taps > 0 ? g_rbt_min_taps : rbt_mink_env;          // b2_debug_set_stacked_min_taps (tests) wins over the environment
-    if (rbt_on && pk.tmap_t && pk.taps >= rbt_mink) return launch_resblock_t(a, st);
+    const int rbt_mink = g_rbt_min_taps > 0 ? g_rbt_min_taps : 5;          // b2_debug_set_stacked_min_taps: the tests run both C = 32 kernels
+    if (pk.tmap_t && pk.taps >= rbt_mink) return launch_resblock_t(a, st);
     RbParams p;
     p.x = a.x; p.acc_src = a.acc_src; p.out32 = a.out32; p.outb = a.outb;
     p.post_w = a.post_w; p.post_b = a.post_b; p.audio = a.audio;
@@ -929,21 +808,9 @@ int launch_resblock(const ResBlockArgs &a, cudaStream_t st) {
     const size_t dbg_n = (size_t)kRbDbgCtas * kRbDbgEvents;
     if (dbg_on && !dbg_buf) B2_CUDA_OK(cudaMalloc(&dbg_buf, dbg_n * 8));
     p.dbg = dbg_on ? dbg_buf : nullptr;
-    static const int nopf = getenv("B2_RB_NOPF") ? atoi(getenv("B2_RB_NOPF")) : 0;
-    static const int noring = getenv("B2_RB_NORING") ? atoi(getenv("B2_RB_NORING")) : 0;
-    p.dbg_flags = (nopf ? 1 : 0) | (noring ? 2 : 0);
-    // look-ahead prefetch distance in CTAs (B2_RB_PFDIST=-1: one resident set, i.e. two CTAs per SM at C = 32, one otherwise).  Measured on the
-    // B200 (profiles/r2f_ab_lookahead_prefetch.json): no gain (nine ResBlock launches 15.67 ms with it, 15.41 ms without) -- the CTA's own
-    // prefetch at its start already hides the HBM latency behind the co-resident CTA.  Off by default.
-    static const int pfd_env = getenv("B2_RB_PFDIST") ? atoi(getenv("B2_RB_PFDIST")) : 0;
-    p.pf_dist = pfd_env >= 0 ? pfd_env : sm_count() * (pk.C == 32 ? 2 : 1);
     if (dbg_on) B2_CUDA_OK(cudaMemsetAsync(dbg_buf, 0, dbg_n * 8, st));
-    // C = 32: four epilogue warps.  B2_RB32_NEW=8 runs the eight-warp variant (warps 4..7 own the odd sub-tiles, 88 registers per thread so
-    // that two CTAs still share an SM).  Measured on the B200 (profiles/r2b_ab_rb32_epilogue_warps.json): SLOWER, 18.3 ms against 15.1 ms for the
-    // nine ResBlock launches of a 1,024-session step -- twice the warps on the same TMEM/shared-memory ports do not shorten the per-conv
-    // epilogue chain, and the single-buffered slab load loses its overlap.  Kept for A/B runs only.
-    static const int new32 = getenv("B2_RB32_NEW") ? atoi(getenv("B2_RB32_NEW")) : 4;
-    const int rc = (pk.C == 32) ? (new32 == 8 ? launch_rb<32, 8, 2>(tm, p, (unsigned)nct, smem, st, 3) : launch_rb<32, 4, 2>(tm, p, (unsigned)nct, smem, st, 0))
+    // C = 32: four epilogue warps (two CTAs share an SM); C = 64 / 128: eight, each with half of a row's columns
+    const int rc = (pk.C == 32) ? launch_rb<32, 4, 2>(tm, p, (unsigned)nct, smem, st, 0)
                    : (pk.C == 64) ? launch_rb<64, 8, 2>(tm, p, (unsigned)nct, smem, st, 1)
                    : launch_rb<128, 8, 2>(tm, p, (unsigned)nct, smem, st, 2);
     if (dbg_on && !rc) {

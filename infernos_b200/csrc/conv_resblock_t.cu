@@ -821,11 +821,7 @@ static int launch_rbt_(const CUtensorMap &tm, const RbtParams &p, unsigned grid,
         B2_CUDA_OK(cudaFuncSetAttribute(k_resblock_t<EPI, DBG, UP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTSmemBytes));
         g_rbt_attr[dev][slot] = true;
     }
-    // B2_RBT_ONE_CTA=1 (analysis runs): ask for more shared memory than two CTAs can share, so that a CTA has the SM to itself
-    static const bool one_cta = getenv("B2_RBT_ONE_CTA") && atoi(getenv("B2_RBT_ONE_CTA")) != 0;
-    const size_t smem = one_cta ? (size_t)120 * 1024 : (size_t)kTSmemBytes;
-    if (one_cta) B2_CUDA_OK(cudaFuncSetAttribute(k_resblock_t<EPI, DBG, UP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    B2_CUDA_OK(launch_k(k_resblock_t<EPI, DBG, UP>, dim3(grid), dim3(192), smem, st, pdl_enabled(), tm, tm_up ? *tm_up : tm, p, g_rbt_dbg));
+    B2_CUDA_OK(launch_k(k_resblock_t<EPI, DBG, UP>, dim3(grid), dim3(192), kTSmemBytes, st, pdl_enabled(), tm, tm_up ? *tm_up : tm, p, g_rbt_dbg));
     B2_LAUNCH_OK("k_resblock_t");
     return 0;
 }

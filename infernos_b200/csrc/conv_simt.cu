@@ -311,7 +311,7 @@ template <int NW>
 __global__ void __launch_bounds__(192) k_chunker_pre(const float *__restrict__ mel, const float *__restrict__ audio,
                                                     const float *__restrict__ wm, const float *__restrict__ bm,
                                                     const float *__restrict__ wa, const float *__restrict__ ba,
-                                                    float *__restrict__ z0, __nv_bfloat16 *__restrict__ z0b, int W) {
+                                                    float *__restrict__ z0, int W) {
     extern __shared__ __align__(16) float smem_f[];
     float *sm = smem_f;                       // [NW][80 * 12]
     float *sa = smem_f + NW * 960;            // [NW][256 * 12]
@@ -354,16 +354,9 @@ __global__ void __launch_bounds__(192) k_chunker_pre(const float *__restrict__ m
 #pragma unroll
         for (int q = 0; q < NW; q++) {
             if (w0 + q >= W) break;
-            if (z0) {
-                float *o = z0 + (long long)(w0 + q) * 12 * 192 + tid;
+            float *o = z0 + (long long)(w0 + q) * 12 * 192 + tid;
 #pragma unroll
-                for (int t = 0; t < 12; t++) o[t * 192] = acc[q][t];
-            }
-            if (z0b) {
-                __nv_bfloat16 *o = z0b + (long long)(w0 + q) * 12 * 192 + tid;
-#pragma unroll
-                for (int t = 0; t < 12; t++) o[t * 192] = __float2bfloat16_rn(lrelu(acc[q][t], 0.01f));
-            }
+            for (int t = 0; t < 12; t++) o[t * 192] = acc[q][t];
         }
         __syncthreads();
     }
@@ -397,7 +390,7 @@ int launch_chunker_in(const float *mel, const float *audio, __nv_bfloat16 *inb, 
 }
 
 int launch_chunker_pre(const float *mel, const float *audio, const float *wm, const float *bm, const float *wa, const float *ba,
-                       float *z0, __nv_bfloat16 *z0b, int W, cudaStream_t st) {
+                       float *z0, int W, cudaStream_t st) {
     if (W <= 0) return 0;
     constexpr int NW = 4;
     static bool attr_set[64] = {};
@@ -410,7 +403,7 @@ int launch_chunker_pre(const float *mel, const float *audio, const float *wm, co
     }
     const int groups = (W + NW - 1) / NW;
     const int cap = sm_count() * 3;
-    k_chunker_pre<NW><<<groups < cap ? groups : cap, 192, smem, st>>>(mel, audio, wm, bm, wa, ba, z0, z0b, W);
+    k_chunker_pre<NW><<<groups < cap ? groups : cap, 192, smem, st>>>(mel, audio, wm, bm, wa, ba, z0, W);
     B2_LAUNCH_OK("k_chunker_pre");
     return 0;
 }

@@ -44,10 +44,9 @@ int launch_normalise(const float *mel, const float *mean, const float *scale, fl
 
 // chunker prologue (HelloSippyRT.py:221-228): conv_pre_m over mel *viewed* as (80,12) and conv_pre_a over audio
 // *viewed* as (256,12), concatenated -> z0 [W][12][192] channels-last (no activation applied).
-// wm packed [3][80][32], wa packed [3][256][160].
-// z0 fp32 and/or z0b = bf16(leaky_relu(z0, 0.01)) (operand of the first chunker upsampler on tensor cores)
+// wm packed [3][80][32], wa packed [3][256][160].  FP32 mode; BF16 mode runs the prologue on tensor cores (launch_chunker_in).
 int launch_chunker_pre(const float *mel, const float *audio, const float *wm, const float *bm, const float *wa, const float *ba,
-                       float *z0, __nv_bfloat16 *z0b, int W, cudaStream_t st);
+                       float *z0, int W, cudaStream_t st);
 // tensor-core form of the prologue: the two `.view`s as ONE bf16 channels-last operand [W][12][384] (audio channels 0..255, mel 256..335, zero pad)
 int launch_chunker_in(const float *mel, const float *audio, __nv_bfloat16 *inb, int W, cudaStream_t st);
 // chunker epilogue (HelloSippyRT.py:235-237): out[w][i] = tanh(audio[w][512+i] * lrelu(post[w][i%8][i/8], 0.01))

@@ -46,10 +46,7 @@ struct UmmaParams {
     int period;       // row period between the windows of a tile (T + pad), or 1<<30
     int tiles_per_win;// ceil(T / 128) when nseg == 1
     int stages;       // B ring depth
-    int mt;           // 128-row M sub-tiles per CTA (tall tiles for the thin layers: 4 at C=32, 2 at C=64)
-    int flags;        // bit 0: skip the generic->async proxy fence after the A-tile barrier (experiment)
     unsigned long long *dbg;   // optional per-CTA phase timestamps (analysis builds)
-    int stagger_ns, sm_count;  // first-wave phase offset between the CTAs that share an SM (0 = off)
     unsigned long long m_period, m_tpw, m_ntiles;   // ceil(2^40 / d) for period, tiles_per_win, ntiles (see fdiv)
 };
 
@@ -78,23 +75,13 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
     // ---- tile coordinates
     int w0, t0;
     if (p.nseg > 1) { w0 = blockIdx.x * p.nseg; t0 = 0; }
-    else { w0 = fdiv(blockIdx.x, p.m_tpw); t0 = (blockIdx.x - w0 * p.tiles_per_win) * 128 * p.mt; }
+    else { w0 = fdiv(blockIdx.x, p.m_tpw); t0 = (blockIdx.x - w0 * p.tiles_per_win) * 128; }
     const int n0 = blockIdx.y * N_TILE;
 
     // Prologue, arranged so that nothing waits for anything it does not need: the TMA thread initialises the barriers and
     // starts streaming weights at once, the producer warps start the first K block of the A tile, warp 5 allocates TMEM;
     // only then does the CTA synchronise.  (what-if runs: this fixed per-CTA cost was 43 % of the thin layers' time.)
     if (threadIdx.x == 0) DBG(0);
-    // CTAs of one wave would otherwise march in lockstep: all in their MMA phase (tensor pipe saturated, HBM idle), then all
-    // in their epilogue (HBM saturated, tensor pipe idle).  Offsetting the co-resident CTAs of the FIRST wave by a fraction of
-    // a CTA lifetime keeps the phases interleaved for the rest of the launch.
-    if (p.stagger_ns > 0 && blockIdx.y == 0) {
-        const int grp = (int)(blockIdx.x / (unsigned)p.sm_count);
-        if (grp > 0 && grp < 4) {
-            const unsigned long long until = gtime() + (unsigned long long)grp * (unsigned long long)p.stagger_ns;
-            while (gtime() < until) __nanosleep(500);
-        }
-    }
     const int total_b = p.nkb * p.taps;
     int b_issued = 0;
     if (warp == 4 && lane == 0) {
@@ -111,7 +98,7 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
         }
     }
     if (warp == 5) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"((uint32_t)(N_TILE * p.mt)) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"((uint32_t)N_TILE) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     const int cshift = (KB == 64) ? 3 : 2;        // 16-byte pieces per row per K block = 1 << cshift
@@ -127,7 +114,7 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
             const int w = w0 + s;
             const bool ok = (t >= 0) && (t < p.T) && (s < p.nseg) && (w < p.W);
             const __nv_bfloat16 *src = ok ? p.in + ((size_t)w * p.T + t) * p.Cin + kb * KB + c * 8 : p.in;
-            cp_async16(sA_u32 + (uint32_t)(((kb * cpr + c) * p.R + r) * 16), src, (ok && !(p.flags & 8)) ? 16u : 0u);
+            cp_async16(sA_u32 + (uint32_t)(((kb * cpr + c) * p.R + r) * 16), src, ok ? 16u : 0u);
         }
     };
     if (warp < 4) {
@@ -159,42 +146,39 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
         if (!p.residual && !p.acc_src && !p.out32) {
             // bf16-only output (conv1 of a pair): a lane already owns 64 contiguous bytes of its row, written as four
             // 128-bit stores; the transpose would only add work (measured 1.16x slower at C=32)
-            for (int sub = 0; sub < p.mt; sub++) {
-                const int m = sub * 128 + warp * 32 + lane;
-                const int s = (p.nseg > 1) ? fdiv(m, p.m_period) : 0;
-                const int t = t0 + (m - s * p.period);
-                const int w = w0 + s;
-                const bool ok = (t < p.T) && (s < p.nseg) && (w < p.W) && !(p.flags & 4);
-                const size_t row_off = ((size_t)w * p.T + t) * p.N + n0;
-#pragma unroll 1
-                for (int c0 = 0; c0 < N_TILE; c0 += 32) {
-                    uint32_t acc[32];
-                    tmem_ld32(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(sub * N_TILE + c0), acc);
-                    if (!ok) continue;
-                    uint4 *op = reinterpret_cast<uint4 *>(p.outb + row_off + c0);
-#pragma unroll
-                    for (int i = 0; i < 4; i++) {
-                        uint32_t pk[4];
-#pragma unroll
-                        for (int e = 0; e < 4; e++) {
-                            const float2 b = __ldg(reinterpret_cast<const float2 *>(p.bias + n0 + c0 + 8 * i + 2 * e));
-                            __nv_bfloat162 h2 = __floats2bfloat162_rn(lrelu_f(__uint_as_float(acc[8 * i + 2 * e]) + b.x, p.outb_slope),
-                                                                      lrelu_f(__uint_as_float(acc[8 * i + 2 * e + 1]) + b.y, p.outb_slope));
-                            pk[e] = *reinterpret_cast<uint32_t *>(&h2);
-                        }
-                        op[i] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-                    }
-                }
-            }
-        } else {
-        float *stg = reinterpret_cast<float *>(sA) + warp * 32 * kStageLd;
-        const int sub_r = lane >> 3, c4 = lane & 7;
-        for (int sub = 0; sub < p.mt; sub++) {
-            const int m = sub * 128 + warp * 32 + lane;
+            const int m = warp * 32 + lane;
             const int s = (p.nseg > 1) ? fdiv(m, p.m_period) : 0;
             const int t = t0 + (m - s * p.period);
             const int w = w0 + s;
-            const int grow_own = ((t < p.T) && (s < p.nseg) && (w < p.W) && !(p.flags & 4)) ? (w * p.T + t) : -1;
+            const bool ok = (t < p.T) && (s < p.nseg) && (w < p.W);
+            const size_t row_off = ((size_t)w * p.T + t) * p.N + n0;
+#pragma unroll 1
+            for (int c0 = 0; c0 < N_TILE; c0 += 32) {
+                uint32_t acc[32];
+                tmem_ld32(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0, acc);
+                if (!ok) continue;
+                uint4 *op = reinterpret_cast<uint4 *>(p.outb + row_off + c0);
+#pragma unroll
+                for (int i = 0; i < 4; i++) {
+                    uint32_t pk[4];
+#pragma unroll
+                    for (int e = 0; e < 4; e++) {
+                        const float2 b = __ldg(reinterpret_cast<const float2 *>(p.bias + n0 + c0 + 8 * i + 2 * e));
+                        __nv_bfloat162 h2 = __floats2bfloat162_rn(lrelu_f(__uint_as_float(acc[8 * i + 2 * e]) + b.x, p.outb_slope),
+                                                                  lrelu_f(__uint_as_float(acc[8 * i + 2 * e + 1]) + b.y, p.outb_slope));
+                        pk[e] = *reinterpret_cast<uint32_t *>(&h2);
+                    }
+                    op[i] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+                }
+            }
+        } else {
+            float *stg = reinterpret_cast<float *>(sA) + warp * 32 * kStageLd;
+            const int sub_r = lane >> 3, c4 = lane & 7;
+            const int m = warp * 32 + lane;
+            const int s = (p.nseg > 1) ? fdiv(m, p.m_period) : 0;
+            const int t = t0 + (m - s * p.period);
+            const int w = w0 + s;
+            const int grow_own = ((t < p.T) && (s < p.nseg) && (w < p.W)) ? (w * p.T + t) : -1;
             int grow[8];
 #pragma unroll
             for (int i = 0; i < 8; i++) grow[i] = __shfl_sync(0xffffffffu, grow_own, i * 4 + sub_r);
@@ -204,7 +188,7 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
                 const float4 bias = __ldg(reinterpret_cast<const float4 *>(p.bias + col));
                 {
                     uint32_t a32[32];
-                    tmem_ld32(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(sub * N_TILE + c0), a32);
+                    tmem_ld32(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0, a32);
 #pragma unroll
                     for (int i = 0; i < 8; i++)
                         *reinterpret_cast<uint4 *>(stg + lane * kStageLd + i * 4) = make_uint4(a32[4 * i], a32[4 * i + 1], a32[4 * i + 2], a32[4 * i + 3]);
@@ -244,7 +228,6 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
                 __syncwarp();
             }
         }
-        }
         if (threadIdx.x == 0) DBG(4);
     } else if (warp == 4) {
         // =========================== B producer (TMA) ===========================
@@ -281,18 +264,17 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
             for (int kb = 0; kb < p.nkb; kb++) {
                 mbar_wait(bar_a_full + 8 * kb, 0);
                 if (kb == 0) DBG(6);
-                if (!(p.flags & 1)) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // cp.async (generic proxy) writes -> UMMA (async proxy) reads
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // cp.async (generic proxy) writes -> UMMA (async proxy) reads
                 for (int j = 0; j < p.taps; j++) {
                     mbar_wait(bar_b_full + 8 * stage, phase);
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     const uint64_t bdesc_s = bdesc0 + (uint64_t)((uint32_t)stage * b_stage_16);
                     const uint32_t a_row = (uint32_t)(kb * (KB / 8) * p.R + j * p.dil);     // in rows (= 16-byte units)
-                    for (int sub = 0; sub < p.mt; sub++)
-                        for (int ks = 0; ks < ksteps; ks++) {
-                            const uint64_t adesc = adesc0 + (uint64_t)(a_row + (uint32_t)(ks * 2 * p.R + sub * 128));
-                            const uint64_t bdesc = bdesc_s + (uint64_t)(ks * 2);
-                            if (!(p.flags & 2)) umma_f16(tb + (uint32_t)(sub * N_TILE), adesc, bdesc, idesc, (accum | (uint32_t)ks) ? 1u : 0u);
-                        }
+                    for (int ks = 0; ks < ksteps; ks++) {
+                        const uint64_t adesc = adesc0 + (uint64_t)(a_row + (uint32_t)(ks * 2 * p.R));
+                        const uint64_t bdesc = bdesc_s + (uint64_t)(ks * 2);
+                        umma_f16(tb, adesc, bdesc, idesc, (accum | (uint32_t)ks) ? 1u : 0u);
+                    }
                     accum = 1;
                     umma_commit(bar_b_empty + 8 * stage);   // frees the B slot when these MMAs retire
                     if (++stage == p.stages) { stage = 0; phase ^= 1; }
@@ -308,7 +290,7 @@ __global__ void __launch_bounds__(kThreads, (N_TILE <= 64) ? 4 : ((N_TILE <= 128
     __syncthreads();
     if (threadIdx.x == 0) DBG(7);
     if (warp == 5) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(N_TILE * p.mt)) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)N_TILE) : "memory");
     }
 }
 
@@ -328,7 +310,6 @@ struct UmmaParams2 {
     int resident;      // all (K-block, tap) weight tiles stay in shared memory
     int rows_per_thr;  // A rows handled by one producer thread per K block
     int iters;         // tiles per CTA, ceil(total_tiles / grid)
-    int mc;            // 2-CTA cluster: each CTA fetches half of every weight tile and multicasts it to both (needs ntiles == 1)
 };
 
 static constexpr int kThreads2 = 320;
@@ -370,11 +351,11 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
     auto ACC_FULL = [&](int a) { return bar0 + 8u * (uint32_t)(2 * NBS + 32 + a); };
     auto ACC_EMPTY = [&](int a) { return bar0 + 8u * (uint32_t)(2 * NBS + 34 + a); };
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * NBS + 36);
-    const uint32_t crank = (PAIR || pp.mc) ? cluster_ctarank() : 0u;
+    const uint32_t crank = PAIR ? cluster_ctarank() : 0u;
 
     if (threadIdx.x == 0) {
         if (smem_u32(smem) & 1023u) __trap();
-        for (int s = 0; s < NBS; s++) { mbar_init(B_FULL(s), 1); mbar_init(B_EMPTY(s), (!PAIR && pp.mc) ? 2 : 1); }     // multicast: both CTAs' MMAs release a slot
+        for (int s = 0; s < NBS; s++) { mbar_init(B_FULL(s), 1); mbar_init(B_EMPTY(s), 1); }
         for (int b = 0; b < 2; b++)
             for (int k = 0; k < 8; k++) { mbar_init(A_FULL(b, k), (PAIR && crank == 0) ? 129 : 128); mbar_init(A_EMPTY(b, k), 1); }
         for (int a = 0; a < 2; a++) { mbar_init(ACC_FULL(a), 1); mbar_init(ACC_EMPTY(a), PAIR ? 8 : 4); }
@@ -389,10 +370,10 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
             asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
         }
     }
-    if (warp == 4 && lane == 0) asm volatile("prefetch.tensormap [%0];" ::"l"(pp.mc ? &tmap_h : &tmap_w) : "memory");
+    if (warp == 4 && lane == 0) asm volatile("prefetch.tensormap [%0];" ::"l"(PAIR ? &tmap_h : &tmap_w) : "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (pp.mc) cluster_sync_all();           // the peer's barriers exist before anything is multicast to them
+    if constexpr (PAIR) cluster_sync_all();  // the peer's barriers exist before anything is multicast to them
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
     // everything above overlapped the previous kernel (PDL); the weight producer (warp 4) reads nothing a kernel writes and goes straight on
@@ -409,8 +390,8 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
         // =========================== epilogue ===========================
         float *stg = sStage + warp * 32 * kStageLd;
         const int sub_r = lane >> 3, c4 = lane & 7;
-        // in multicast mode both CTAs of a cluster run the same number of tiles (the weight ring is shared): tiles past the end are
-        // dummies whose rows are all masked (w >= W)
+        // both CTAs of a pair run the same number of tiles (the MMAs are shared): tiles past the end are dummies whose rows are
+        // all masked (w >= W)
         // The fp32 residual / MRF-sum rows a tile's epilogue will add come from HBM (the tensors are larger than L2): they are pulled
         // into L2 one TILE ahead (lane = row, one 128-byte line per 32-column piece), so that the register prefetch one PIECE ahead
         // only has to cover an L2 hit.  No registers are held across the wait.
@@ -433,7 +414,7 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
         l2_prefetch_tile((int)blockIdx.x);
         for (int it = 0; it < pp.iters; ++it) {
             const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-            if (!pp.mc && tile >= pp.total_tiles) break;
+            if (!PAIR && tile >= pp.total_tiles) break;
             l2_prefetch_tile(tile + (int)gridDim.x);
             int w0, t0, n0;
             tile_coords(tile, w0, t0, n0);
@@ -442,7 +423,7 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
             const int s = (p.nseg > 1) ? fdiv(m, p.m_period) : 0;
             const int t = t0 + (m - s * p.period);
             const int w = w0 + s;
-            const int grow_own = ((t < p.T) && (s < p.nseg) && (w < p.W) && !(p.flags & 4)) ? (w * p.T + t) : -1;
+            const int grow_own = ((t < p.T) && (s < p.nseg) && (w < p.W)) ? (w * p.T + t) : -1;
             int grow[8];
 #pragma unroll
             for (int i = 0; i < 8; i++) grow[i] = __shfl_sync(0xffffffffu, grow_own, i * 4 + sub_r);
@@ -550,32 +531,21 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
                 int stage = 0; uint32_t phase = 0;
                 for (int it = 0; it < pp.iters; ++it) {
                     const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-                    if (!pp.mc && tile >= pp.total_tiles) break;
+                    if (!PAIR && tile >= pp.total_tiles) break;
                     int w0, t0, n0;
                     tile_coords(tile, w0, t0, n0);
                     for (int kb = 0; kb < p.nkb; kb++)
                         for (int j = 0; j < p.taps; j++) {
-                            if (p.flags & 32) continue;      // what-if: no weight ring at all (no loads, no barrier traffic)
                             mbar_wait(B_EMPTY(stage), phase ^ 1);
-                            if (p.flags & 16) {      // what-if: no weight traffic at all (the MMAs read whatever the ring holds)
-                                if (!PAIR || crank == 0) mbar_arrive(B_FULL(stage));
-                                if (++stage == p.stages) { stage = 0; phase ^= 1; }
-                                continue;
-                            }
                             if constexpr (PAIR) {
                                 // my half of the tile into MY shared memory; the bytes of both halves are counted on the leader's barrier
                                 if (crank == 0) mbar_expect_tx(B_FULL(stage), 2 * b_tile_bytes);
                                 tma_load_3d_2sm(smem_u32(sB + (size_t)stage * b_tile_bytes), &tmap_h, mapa_u32(B_FULL(stage), 0u), kb * KB,
                                                 n0 + (int)crank * (N_TILE / 2), j);
-                                if (++stage == p.stages) { stage = 0; phase ^= 1; }
-                                continue;
-                            }
-                            mbar_expect_tx(B_FULL(stage), b_tile_bytes);
-                            if (pp.mc)       // my half of the tile, into both CTAs: L2 serves every weight byte once per cluster
-                                tma_load_3d_mc(smem_u32(sB + (size_t)stage * b_tile_bytes) + crank * (b_tile_bytes / 2), &tmap_h, B_FULL(stage),
-                                               kb * KB, n0 + (int)crank * (N_TILE / 2), j, (uint16_t)3);
-                            else
+                            } else {
+                                mbar_expect_tx(B_FULL(stage), b_tile_bytes);
                                 tma_load_3d(smem_u32(sB + (size_t)stage * b_tile_bytes), &tmap_w, B_FULL(stage), kb * KB, n0, j);
+                            }
                             if (++stage == p.stages) { stage = 0; phase ^= 1; }
                         }
                 }
@@ -608,7 +578,7 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
             if (pp.resident) { mbar_wait(B_FULL(0), 0); }
             for (int it = 0; it < pp.iters; ++it) {
                 const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-                if (!pp.mc && tile >= pp.total_tiles) break;
+                if (!PAIR && tile >= pp.total_tiles) break;
                 const int acc = it & 1, use = it >> 1;
                 const int abuf = (pp.nA == 2) ? (it & 1) : 0, ause = (pp.nA == 2) ? (it >> 1) : it;
                 if constexpr (PAIR) mbar_wait_cluster(ACC_EMPTY(acc), (uint32_t)((use & 1) ^ 1));
@@ -622,25 +592,23 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
                     if constexpr (PAIR) mbar_wait_cluster(A_FULL(abuf, kb), (uint32_t)(ause & 1));
                     else mbar_wait(A_FULL(abuf, kb), (uint32_t)(ause & 1));
                     if (kb == 0) PDBG(3);
-                    if (!(p.flags & 1)) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                     for (int j = 0; j < p.taps; j++) {
                         uint64_t bdesc_s;
                         if (pp.resident) bdesc_s = bdesc0 + (uint64_t)((uint32_t)(kb * p.taps + j) * b_tile_16);
                         else {
-                            if (!(p.flags & 32)) mbar_wait(B_FULL(stage), phase);
+                            mbar_wait(B_FULL(stage), phase);
                             bdesc_s = bdesc0 + (uint64_t)((uint32_t)stage * b_tile_16);
                         }
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                         const uint32_t a_row = (uint32_t)(kb * (KB / 8) * p.R + j * p.dil);
                         for (int ks = 0; ks < ksteps; ks++) {
                             if constexpr (PAIR) umma_f16_2cta(tmem_acc, adesc_t + (uint64_t)(a_row + (uint32_t)(ks * 2 * p.R)), bdesc_s + (uint64_t)(ks * 2), idesc, accum);
-                            else if (!(p.flags & 2)) umma_f16(tmem_acc, adesc_t + (uint64_t)(a_row + (uint32_t)(ks * 2 * p.R)), bdesc_s + (uint64_t)(ks * 2), idesc, accum);
+                            else umma_f16(tmem_acc, adesc_t + (uint64_t)(a_row + (uint32_t)(ks * 2 * p.R)), bdesc_s + (uint64_t)(ks * 2), idesc, accum);
                             accum = 1;
                         }
                         if (!pp.resident) {
-                            if (p.flags & 32) { if (++stage == p.stages) { stage = 0; phase ^= 1; } continue; }
                             if constexpr (PAIR) umma_commit_2cta(B_EMPTY(stage), (uint16_t)3);
-                            else if (pp.mc) umma_commit_mc(B_EMPTY(stage), (uint16_t)3);
                             else umma_commit(B_EMPTY(stage));
                             if (++stage == p.stages) { stage = 0; phase ^= 1; }
                         }
@@ -664,7 +632,7 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
         const int r_first = ptid >> cshift, c = ptid & (cpr - 1);
         for (int it = 0; it < pp.iters; ++it) {
             const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-            if (!pp.mc && tile >= pp.total_tiles) break;
+            if (!PAIR && tile >= pp.total_tiles) break;
             int w0, t0, n0;
             tile_coords(tile, w0, t0, n0);
             const int abuf = (pp.nA == 2) ? (it & 1) : 0, ause = (pp.nA == 2) ? (it >> 1) : it;
@@ -688,7 +656,7 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
                     const int r = r_first + i * rstep;
                     if (r < p.R) {
                         const __nv_bfloat16 *src = grow[i] >= 0 ? p.in + (size_t)grow[i] * p.Cin + kb * KB + c * 8 : p.in;
-                        cp_async16(sA_u32 + (uint32_t)(((kb * cpr + c) * p.R + r) * 16), src, (grow[i] >= 0 && !(p.flags & 8)) ? 16u : 0u);
+                        cp_async16(sA_u32 + (uint32_t)(((kb * cpr + c) * p.R + r) * 16), src, grow[i] >= 0 ? 16u : 0u);
                     }
                 }
                 cp_async_arrive_noinc(A_FULL(abuf, kb));
@@ -699,7 +667,7 @@ __global__ void __launch_bounds__(kThreads2, MINB) k_conv_umma_p(const __grid_co
 
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (pp.mc) cluster_sync_all();           // nobody leaves while the peer may still arrive on this CTA's barriers
+    if constexpr (PAIR) cluster_sync_all();  // nobody leaves while the peer may still arrive on this CTA's barriers
     if (warp == 5) {
         if constexpr (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * N_TILE)) : "memory");
         else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * N_TILE)) : "memory");
@@ -714,28 +682,9 @@ static EncodeTiledFn g_encode = nullptr;
 static std::mutex g_init_mu;
 static bool g_attr_set[64][4] = {};
 
-// Stage 0 (C = 256, T = 48) is bound by re-streaming the weights from L2 for every 128-row tile (k x 128 KB per two windows).
-// Experiment (B2_UMMA_TALL256=1): its ResBlock convs as 256-row tiles (two M sub-tiles per weight tile, up to five windows packed
-// per tile) of 128 output channels in the one-tile-per-CTA kernel, i.e. half the weight bytes per FLOP.  Measured on B200: correct,
-// but 5 % SLOWER end to end (26.3 vs 25.0 ms per step) -- at one CTA per SM its load / MMA / epilogue phases do not overlap, which
-// costs more than the weight traffic saves -- so the persistent pipelined kernel stays the default for these layers.
-static bool tall256() {
-    static const bool on = getenv("B2_UMMA_TALL256") && atoi(getenv("B2_UMMA_TALL256")) != 0;
-    return on;
-}
-static bool is_tall256(const Layer &l) { return tall256() && l.Cin == 256 && l.Cout == 256; }
-
 static int n_tile_for(const Layer &l) {
-    if (is_tall256(l)) return 128;
     if (l.Cout >= 256) return (l.Cin >= 512) ? 128 : 256;
     return l.Cout;     // 32, 64, 128
-}
-
-static int umma_flags() {
-    // bit 0: skip the proxy fence; what-if switches for profiling only (results are wrong with them):
-    // bit 1: issue no MMAs, bit 2: epilogue touches no global memory, bit 3: A producer loads nothing, bit 4: no weight loads, bit 5: no weight ring (neither loads nor its barriers / commits) (persistent kernel)
-    static const int f = (getenv("B2_NO_PROXY_FENCE") ? 1 : 0) | (getenv("B2_UMMA_WHATIF") ? atoi(getenv("B2_UMMA_WHATIF")) << 1 : 0);
-    return f;
 }
 
 int umma_init() {
@@ -777,7 +726,7 @@ int umma_prepare_layer(Layer &l) {
         l.tmap_q = tq;
     }
     if (nt == 256 && l.Cout == 256) {
-        // the persistent kernel's 2-CTA multicast mode: the same tensor with a box of half the tile's rows
+        // the CTA pair of the persistent kernel: the same tensor with a box of half the tile's rows (each CTA loads its half)
         CUtensorMap *th = new CUtensorMap();
         cuuint32_t boxh[3] = {(cuuint32_t)KB, (cuuint32_t)(nt / 2), 1};
         r = g_encode(th, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, (void *)l.wbf, gdim, gstr, boxh, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
@@ -807,6 +756,7 @@ static int launch_nt(const CUtensorMap &tm, const UmmaParams &p, dim3 grid, size
     return 0;
 }
 
+// the thin layers (Cout <= 128): one 128-row tile per CTA, many CTAs per SM
 static int launch_conv_umma_v1(const UmmaConvArgs &a, cudaStream_t st) {
     const Layer &l = *a.layer;
     if (!l.tmap || !l.wbf) return set_error("conv_umma: layer has no tensor-core weights (context not in B2_MODE_BF16?)");
@@ -815,9 +765,6 @@ static int launch_conv_umma_v1(const UmmaConvArgs &a, cudaStream_t st) {
     UmmaParams p;
     p.in = a.in; p.bias = l.bias; p.residual = a.residual; p.acc_src = a.acc_src; p.out32 = a.out32; p.outb = a.outb;
     p.outb_slope = a.outb_slope; p.div = a.div;
-    p.flags = umma_flags();
-    static const int stagger_env = getenv("B2_UMMA_STAGGER_NS") ? atoi(getenv("B2_UMMA_STAGGER_NS")) : 0;
-    p.stagger_ns = stagger_env; p.sm_count = sm_count();
     static const bool dbg_on = getenv("B2_UMMA_DBG") != nullptr;
     static unsigned long long *dbg_buf = nullptr;
     if (dbg_on && !dbg_buf) cudaMalloc(&dbg_buf, 8192 * 8 * 8);
@@ -827,29 +774,17 @@ static int launch_conv_umma_v1(const UmmaConvArgs &a, cudaStream_t st) {
     p.KB = l.Cin >= 64 ? 64 : 32;
     p.nkb = l.Cin / p.KB;
     const int nt = n_tile_for(l);
-    // tall tiles for the thin layers: the per-CTA latency chain (load -> MMA -> epilogue) is amortised over mt x 128 rows
-    static const int mt_env = getenv("B2_UMMA_MT") ? atoi(getenv("B2_UMMA_MT")) : 0;
-    p.mt = 1;
-    if (a.T >= 128 && l.Cout == nt) {
-        static const int mt32 = getenv("B2_UMMA_MT32") ? atoi(getenv("B2_UMMA_MT32")) : 4;
-        static const int mt64 = getenv("B2_UMMA_MT64") ? atoi(getenv("B2_UMMA_MT64")) : 1;
-        int want = (l.Cin <= 32 && nt <= 32) ? mt32 : ((l.Cin <= 64 && nt <= 64) ? mt64 : 1);
-        if (mt_env > 0) want = std::min(mt_env, want);
-        while (want > 1 && 128 * want > ((a.T + 127) / 128) * 128) want >>= 1;
-        p.mt = want;
-    }
-    if (is_tall256(l)) p.mt = 2;
-    p.R = (128 * p.mt + (l.taps - 1) * l.dil) | 1;
+    p.R = (128 + (l.taps - 1) * l.dil) | 1;
     unsigned mtiles;
-    if (a.T < 128 * p.mt) {
-        // short windows: several per tile, `pad` zero rows apart (the thin layers never get here with mt > 1)
+    if (a.T < 128) {
+        // short windows: several per tile, `pad` zero rows apart
         const int G = l.pad;
-        p.nseg = std::max(1, (128 * p.mt + G) / (a.T + G));
+        p.nseg = std::max(1, (128 + G) / (a.T + G));
         p.period = a.T + G;
         p.tiles_per_win = 1;
         mtiles = (unsigned)cdiv(a.W, p.nseg);
     } else {
-        p.nseg = 1; p.period = 1 << 30; p.tiles_per_win = cdiv(a.T, 128 * p.mt);
+        p.nseg = 1; p.period = 1 << 30; p.tiles_per_win = cdiv(a.T, 128);
         mtiles = (unsigned)((long long)a.W * p.tiles_per_win);
     }
     p.m_period = ((1ull << 40) + (unsigned long long)p.period - 1) / (unsigned long long)p.period;
@@ -858,12 +793,8 @@ static int launch_conv_umma_v1(const UmmaConvArgs &a, cudaStream_t st) {
     const size_t a_bytes = (std::max<size_t>((size_t)p.R * l.Cin * 2, (size_t)kStageBytes) + 15) & ~(size_t)15;
     const size_t b_stage = (size_t)nt * p.KB * 2;
     const size_t tail_bytes = (2 * 16 + kMaxKB + 1) * 8 + 16;
-    // Weight ring depth.  On the thin layers a tap is little MMA work (0.3 us) against a ~1 us TMA round trip, so the ring
-    // is made deep enough to have every tap of the layer in flight at once; the wide layers keep 4 stages (smem).
-    static const int st32 = getenv("B2_UMMA_STAGES32") ? atoi(getenv("B2_UMMA_STAGES32")) : 4;
-    static const int st64 = getenv("B2_UMMA_STAGES64") ? atoi(getenv("B2_UMMA_STAGES64")) : 4;
-    int stages = (nt <= 32 && l.Cin <= 32) ? st32 : ((nt <= 64 && l.Cin <= 64) ? st64 : 4);
-    stages = std::max(2, std::min(stages, 16));
+    // weight ring: four stages, fewer where shared memory runs out or the layer has fewer (K block, tap) tiles
+    int stages = 4;
     while (stages > 2 && stages * b_stage + a_bytes + tail_bytes > 200 * 1024) stages--;
     const int total_b = p.nkb * l.taps;
     if (stages > total_b) stages = std::max(1, total_b);
@@ -876,8 +807,7 @@ static int launch_conv_umma_v1(const UmmaConvArgs &a, cudaStream_t st) {
     switch (nt) {
         case 32: rc = launch_nt<32>(tm, p, grid, smem, st, 0); break;
         case 64: rc = launch_nt<64>(tm, p, grid, smem, st, 1); break;
-        case 128: rc = launch_nt<128>(tm, p, grid, smem, st, 2); break;
-        default: rc = launch_nt<256>(tm, p, grid, smem, st, 3); break;
+        default: rc = launch_nt<128>(tm, p, grid, smem, st, 2); break;
     }
     if (dbg_on && !rc) {
         cudaStreamSynchronize(st);
@@ -900,15 +830,15 @@ static int launch_conv_umma_v1(const UmmaConvArgs &a, cudaStream_t st) {
             d[6] += (double)(r[7] - r[4]);   // teardown sync
             d[7] += (double)(r[7] - r[0]);   // CTA lifetime
         }
-        if (cnt) fprintf(stderr, "[umma dbg] N=%d Cin=%d taps=%d dil=%d mt=%d grid=%u res=%d out32=%d | ns: setup %.0f, A-issue %.0f, A-landed %.0f, mma-loop %.0f, commit->epi %.0f, epilogue %.0f, teardown %.0f, lifetime %.0f | span %.1f us for %d CTAs\n",
-                         nt, l.Cin, l.taps, l.dil, p.mt, grid.x, a.residual != nullptr, a.out32 != nullptr, d[0] / cnt, d[1] / cnt, d[2] / cnt, d[3] / cnt, d[4] / cnt, d[5] / cnt, d[6] / cnt, d[7] / cnt,
+        if (cnt) fprintf(stderr, "[umma dbg] N=%d Cin=%d taps=%d dil=%d grid=%u res=%d out32=%d | ns: setup %.0f, A-issue %.0f, A-landed %.0f, mma-loop %.0f, commit->epi %.0f, epilogue %.0f, teardown %.0f, lifetime %.0f | span %.1f us for %d CTAs\n",
+                         nt, l.Cin, l.taps, l.dil, grid.x, a.residual != nullptr, a.out32 != nullptr, d[0] / cnt, d[1] / cnt, d[2] / cnt, d[3] / cnt, d[4] / cnt, d[5] / cnt, d[6] / cnt, d[7] / cnt,
                          (double)(tmax - tmin) / 1e3, cnt);
     }
     return rc;
 }
 
 
-static int g_occ2[64][6] = {};
+static int g_occ2[64][5] = {};
 
 template <int NT, int MINB, bool PAIR = false>
 static int launch_nt2(const CUtensorMap &tm, const CUtensorMap *tm_half, UmmaParams2 &p, size_t smem, cudaStream_t st, int slot) {
@@ -924,13 +854,6 @@ static int launch_nt2(const CUtensorMap &tm, const CUtensorMap *tm_half, UmmaPar
     occ = std::max(1, std::min(occ, std::min(MINB, 512 / (2 * NT))));
     int grid = std::min(p.total_tiles, sm_count() * occ);
     if (PAIR) grid = std::min((p.total_tiles + 1) & ~1, (sm_count() * occ) & ~1);      // whole pairs; a tile past the end is a dummy (all rows masked)
-    // Experiment (B2_UMMA_MULTICAST=1): weight multicast in 2-CTA clusters for the C=256 ResBlock convs (one N tile, weights streamed:
-    // 0.8-2.9 GB of L2 reads per launch otherwise) -- each CTA fetches half of every weight tile and TMA-multicasts it to both.
-    // Measured on B200: correct, and NO faster (23.92 vs 23.93 ms per step); a 2-deep instead of 3-deep weight ring costs only 2.6 %
-    // as well, so these launches are bound neither by L2 reads nor by weight-fetch latency.  Off by default.
-    static const bool mc_on = getenv("B2_UMMA_MULTICAST") && atoi(getenv("B2_UMMA_MULTICAST")) != 0;
-    p.mc = PAIR ? 2 : ((mc_on && tm_half && p.ntiles == 1 && !p.resident && grid >= 2 && occ == 1) ? 1 : 0);
-    if (p.mc) grid &= ~1;
     p.iters = cdiv(p.total_tiles, grid);
     static const bool pdbg_on = getenv("B2_UMMA_PDBG") != nullptr;
     static unsigned long long *pdbg_buf = nullptr;
@@ -968,7 +891,7 @@ static int launch_nt2(const CUtensorMap &tm, const CUtensorMap *tm_half, UmmaPar
                              d[0] / cnt, d[1] / cnt, d[2] / cnt, d[3] / cnt, d[4] / cnt, d[5] / cnt, d[6] / cnt, d[7] / cnt, cnt);
         }
     };
-    if (!p.mc) {
+    if constexpr (!PAIR) {
         B2_CUDA_OK(launch_k(k_conv_umma_p<NT, MINB, PAIR>, dim3(grid), dim3(kThreads2), smem, st, pdl_enabled(), tm, tm, p));
         B2_LAUNCH_OK("k_conv_umma_p");
         report();
@@ -981,9 +904,9 @@ static int launch_nt2(const CUtensorMap &tm, const CUtensorMap *tm_half, UmmaPar
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = (PAIR && pdl_enabled()) ? 2 : 1;
+    cfg.attrs = at; cfg.numAttrs = pdl_enabled() ? 2 : 1;
     B2_CUDA_OK(cudaLaunchKernelEx(&cfg, k_conv_umma_p<NT, MINB, PAIR>, tm, *tm_half, (const UmmaParams2)p));
-    B2_LAUNCH_OK(PAIR ? "k_conv_umma_p (cta_group::2)" : "k_conv_umma_p (2-CTA multicast)");
+    B2_LAUNCH_OK("k_conv_umma_p (cta_group::2)");
     report();
     return 0;
 }
@@ -991,11 +914,10 @@ static int launch_nt2(const CUtensorMap &tm, const CUtensorMap *tm_half, UmmaPar
 int launch_conv_umma(const UmmaConvArgs &a, cudaStream_t st) {
     // Two kernels, chosen per layer from the round-1 launch lists (profiles/): the persistent pipelined kernel wins on the
     // wide layers (stage 0, the upsamplers); the one-tile-per-CTA kernel with many co-resident CTAs wins on the thin ones,
-    // where a tile is too little work to amortise a pipeline hand-off.  B2_UMMA_V1 / B2_UMMA_V2 force one of them.
-    static const bool force_v1 = getenv("B2_UMMA_V1") != nullptr, force_v2 = getenv("B2_UMMA_V2") != nullptr;
+    // where a tile is too little work to amortise a pipeline hand-off.
     const Layer &l = *a.layer;
     const bool wide = l.Cin >= 256 || l.Cout > l.Cin;
-    if (force_v1 || (!force_v2 && (!wide || is_tall256(l)))) return launch_conv_umma_v1(a, st);
+    if (!wide) return launch_conv_umma_v1(a, st);
     if (!l.tmap || !l.wbf) return set_error("conv_umma: layer has no tensor-core weights (context not in B2_MODE_BF16?)");
     if (a.W <= 0 || a.T <= 0) return 0;
     if ((l.taps - 1) * l.dil != 2 * l.pad) return set_error("conv_umma: only 'same' convolutions are supported");
@@ -1003,10 +925,8 @@ int launch_conv_umma(const UmmaConvArgs &a, cudaStream_t st) {
     UmmaParams &p = pp.b;
     p.in = a.in; p.bias = l.bias; p.residual = a.residual; p.acc_src = a.acc_src; p.out32 = a.out32; p.outb = a.outb;
     p.outb_slope = a.outb_slope; p.div = a.div;
-    p.flags = umma_flags();
     p.W = a.W; p.T = a.T; p.Cin = l.Cin; p.N = l.Cout; p.taps = l.taps; p.dil = l.dil; p.pad = l.pad;
-    p.mt = 1;
-    p.dbg = nullptr; p.stagger_ns = 0; p.sm_count = sm_count();
+    p.dbg = nullptr;
     p.R = (128 + (l.taps - 1) * l.dil) | 1;
     p.KB = l.Cin >= 64 ? 64 : 32;
     p.nkb = l.Cin / p.KB;
@@ -1033,9 +953,7 @@ int launch_conv_umma(const UmmaConvArgs &a, cudaStream_t st) {
     // The C = 256 layers (stage 0's 18 ResBlock convs, 4 ms of the step) run as CTA pairs on `tcgen05.mma.cta_group::2` (see k_conv_umma_p, PAIR):
     // the single-CTA launches ran at the SM's shared-memory bandwidth, not at the tensor pipe's pace -- per k = 11 tile 2.1 MB of operand reads
     // + 1.4 MB of TMA writes + 0.35 MB of A / epilogue traffic = 30k cycles at 128 B/cycle against 32.4k measured and 22.5k of tensor-pipe time.
-    // B2_UMMA_PAIR=0 keeps the single-CTA kernel.
-    static const bool pair_on = !(getenv("B2_UMMA_PAIR") && atoi(getenv("B2_UMMA_PAIR")) == 0);
-    const bool pair = pair_on && nt == 256 && pp.ntiles == 1 && l.tmap_half && pp.total_tiles >= 2 && p.KB == 64 && l.Cin >= 256;    // not upsampler 2 (128 -> 256: 0.38 vs 0.35 ms as a pair, launch list r3)
+    const bool pair = nt == 256 && pp.ntiles == 1 && l.tmap_half && pp.total_tiles >= 2 && p.KB == 64 && l.Cin >= 256;    // not upsampler 2 (128 -> 256: 0.38 vs 0.35 ms as a pair, launch list r3)
     const size_t b_tile = (size_t)(pair ? nt / 2 : nt) * p.KB * 2;
     const size_t fixed = kStageBytes + (pair ? 56 : 48) * 8 + 16;
     const size_t budget = 225 * 1024;
@@ -1044,28 +962,15 @@ int launch_conv_umma(const UmmaConvArgs &a, cudaStream_t st) {
     pp.resident = (!pair && pp.ntiles == 1 && all_w + 2 * a_bytes + fixed <= 72 * 1024) ? 1 : 0;
     size_t b_bytes;
     if (pp.resident) { b_bytes = all_w; p.stages = 0; pp.nA = 2; }
-    else if (pair) {
-        // 16 KB per stage and CTA: two A buffers where four stages still fit beside them, else one A buffer; then as deep a ring as fits (at most 8)
-        static const int prefer_na = getenv("B2_UMMA_P_NA") ? atoi(getenv("B2_UMMA_P_NA")) : 0;
-        static const int st_cap = getenv("B2_UMMA_P_STAGES") ? atoi(getenv("B2_UMMA_P_STAGES")) : 8;
-        int stages = 8;
-        pp.nA = 2;
-        if (prefer_na == 1 || (prefer_na == 0 && 4 * b_tile + 2 * a_bytes + fixed > budget)) pp.nA = 1;
-        while (stages > 2 && stages * b_tile + pp.nA * a_bytes + fixed > budget) stages--;
-        stages = std::max(1, std::min(stages, std::min(st_cap, 8)));
-        p.stages = std::min(stages, std::max(1, p.nkb * l.taps));
-        b_bytes = p.stages * b_tile;
-    } else {
+    else {
         // Streamed weights need a DEEP ring before a second A buffer: an N=256 tile consumes 64 B of weights per cycle, i.e. 4 x 32 KB
         // in flight at ~1 us of L2 latency.  (B2_UMMA_PDBG: with two A buffers and a 2-deep ring the MMA loop of the C=256 layers ran
         // at 1.8x its tensor-pipe time, with one A buffer -- K blocks recycled as their MMAs retire -- and 3-4 stages at 1.4x.)
-        static const int prefer_na = getenv("B2_UMMA_P_NA") ? atoi(getenv("B2_UMMA_P_NA")) : 0;      // 0 = policy below
-        int stages = 4;
-        pp.nA = 2;
-        if (prefer_na == 1 || (prefer_na == 0 && stages * b_tile + 2 * a_bytes + fixed > budget)) pp.nA = 1;
+        // So: two A buffers where four stages still fit beside them, else one; then as deep a ring as fits, at most 4 stages
+        // (8 for a pair, whose stages are half a tile: 16 KB per CTA).
+        int stages = pair ? 8 : 4;
+        pp.nA = (4 * b_tile + 2 * a_bytes + fixed > budget) ? 1 : 2;
         while (stages > 2 && stages * b_tile + pp.nA * a_bytes + fixed > budget) stages--;
-        static const int st_cap = getenv("B2_UMMA_P_STAGES") ? atoi(getenv("B2_UMMA_P_STAGES")) : 4;     // analysis: fewer weight tiles in flight
-        stages = std::max(1, std::min(stages, st_cap));
         p.stages = std::min(stages, std::max(1, p.nkb * l.taps));
         b_bytes = p.stages * b_tile;
     }
@@ -1076,16 +981,10 @@ int launch_conv_umma(const UmmaConvArgs &a, cudaStream_t st) {
     switch (nt) {
         case 32: return launch_nt2<32, 3>(tm, nullptr, pp, smem, st, 0);
         case 64: return launch_nt2<64, 2>(tm, nullptr, pp, smem, st, 1);
-        case 128: {
-            // Experiment (B2_UMMA_P128_OCC=2): two CTAs per SM for upsampler 3 (2.0 GB of traffic in 0.88 ms = 2.3 TB/s).  Measured on
-            // B200: SLOWER (conv_tc class 7.53 -> 9.61 ms per step): the 96-register cap spills the epilogue.  Off by default.
-            static const int occ128 = getenv("B2_UMMA_P128_OCC") ? atoi(getenv("B2_UMMA_P128_OCC")) : 1;
-            if (occ128 >= 2 && smem <= 100 * 1024) return launch_nt2<128, 2>(tm, nullptr, pp, smem, st, 4);
-            return launch_nt2<128, 1>(tm, nullptr, pp, smem, st, 2);
-        }
+        case 128: return launch_nt2<128, 1>(tm, nullptr, pp, smem, st, 2);
         default:
-            if (pair) return launch_nt2<256, 1, true>(tm, th, pp, smem, st, 5);
-            return launch_nt2<256, 1>(tm, th, pp, smem, st, 3);
+            if (pair) return launch_nt2<256, 1, true>(tm, th, pp, smem, st, 4);
+            return launch_nt2<256, 1>(tm, nullptr, pp, smem, st, 3);
     }
 }
 

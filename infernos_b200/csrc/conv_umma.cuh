@@ -48,13 +48,12 @@ bool resblock_supported(int C, int taps);
 int resblock_pack(const Layer *const conv1[3], const Layer *const conv2[3], ResBlockPack &out, std::vector<void *> &allocs, size_t &bytes);
 void resblock_free(ResBlockPack &p);
 int launch_resblock(const ResBlockArgs &a, cudaStream_t st);
-// C = 32: four output time steps stacked into the MMA's N dimension (conv_resblock_t.cu); launch_resblock dispatches to it (B2_RB_T=0: never)
+// C = 32: four output time steps stacked into the MMA's N dimension (conv_resblock_t.cu); launch_resblock dispatches to it
 bool resblock_t_supported(int C, int taps, const int dil[3]);
 int resblock_t_pack(ResBlockPack &out, std::vector<void *> &allocs, size_t &bytes);
 void resblock_t_free(ResBlockPack &p);
 int resblock_t_plan(int k, const int dil[3], int T, bool post, int &S, int &H, int &V, int &tiles, int off[3], int lim[3], bool align4 = false);
 int launch_resblock_t(const ResBlockArgs &a, cudaStream_t st);
-bool resblock_t_enabled();          // B2_RB_T != 0
 extern int g_rbt_min_taps;          // > 0: smallest tap count launch_resblock hands to the stacked-output kernel (b2_debug_set_stacked_min_taps)
 // builds the TMA descriptor of a layer's bf16 weights; called once from b2_weights_finalize
 int umma_prepare_layer(Layer &l);

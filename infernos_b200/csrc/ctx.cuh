@@ -44,7 +44,7 @@ struct Workspace {
     __nv_bfloat16 *c0b = nullptr;                      // [F][512] bf16 (BF16 mode)
     __nv_bfloat16 *hb = nullptr, *yb = nullptr, *rb = nullptr, *sb = nullptr;       // [F*8192] bf16
     float *audio = nullptr;                            // [F*256]
-    // chunker, per window
+    // chunker, per window (z0, z1, zy, z3: FP32 mode only)
     float *z0 = nullptr, *z1 = nullptr, *z2 = nullptr, *zy = nullptr, *z3 = nullptr, *post = nullptr;
     __nv_bfloat16 *win_norm_b = nullptr;               // [F][128] bf16, bins 80..127 zero (BF16 mode)
     __nv_bfloat16 *z0b = nullptr, *z1b = nullptr, *z2b = nullptr, *zyb = nullptr;   // chunker operands (BF16 mode)
@@ -98,7 +98,6 @@ struct b2_ctx {
     b2::Layer c_pre_tc;
     __nv_bfloat16 *c_post_wbf = nullptr;               // [256][512] bf16: W[n][j * 64 + ci] = post_conv.weight[n][ci][j]
     void *c_post_tmA = nullptr, *c_post_tmB = nullptr; // CUtensorMap: A over z3b with a 24-row (1536-element) stride, B over c_post_wbf
-    bool chunker_tc = false;
 
     // SpeechT5 decoder post-net (optional; SURVEY 8 f3): five k5 convs, batch norm folded in
     bool has_postnet = false;

@@ -223,10 +223,8 @@ static int finalize(b2_ctx *c) {
         if (!(w = find(c->chk_raw, "conv_pre_a.weight", {160, 256, 3})) || !(b = find(c->chk_raw, "conv_pre_a.bias", {160}))) return 1;
         if (pack_conv(c, tmp, *w, *b, 1, 1, 1, false)) return 1;
         c->cwa = tmp.w32; c->cba = tmp.bias;
-        static const bool chk_tc = !(getenv("B2_CHUNKER_TC") && atoi(getenv("B2_CHUNKER_TC")) == 0);
-        c->chunker_tc = bf && chk_tc;
         if (!(w = find(c->chk_raw, "upsampler.0.weight", {192, 128, 8})) || !(b = find(c->chk_raw, "upsampler.0.bias", {128}))) return 1;
-        if (c->chunker_tc) {
+        if (bf) {
             // the prologue's output is padded from 192 to 256 channels (one N = 256 tile), so the first upsampler takes 256 input channels
             HostTensor wp;
             wp.shape = {256, 128, 8};
@@ -242,7 +240,7 @@ static int finalize(b2_ctx *c) {
         if (pack_conv(c, c->c_res2, *w, *b, 3, 3, 1, bf)) return 1;
         if (!(w = find(c->chk_raw, "post_conv.weight", {256, 64, 8})) || !(b = find(c->chk_raw, "post_conv.bias", {256}))) return 1;
         if (pack_conv(c, c->c_post, *w, *b, 1, 0, 24, false)) return 1;
-        if (c->chunker_tc) {
+        if (bf) {
             // post_conv as a GEMM: row (window, t) of the operand is the 8 x 64 = 512 contiguous bf16 of z3b rows 24t .. 24t+7
             std::vector<float> q((size_t)256 * 512);
             for (int n = 0; n < 256; n++)
@@ -312,10 +310,9 @@ static int finalize(b2_ctx *c) {
     if (dev_alloc(c, &ws.h, F * 8192) || dev_alloc(c, &ws.r, F * 8192) || dev_alloc(c, &ws.s0, F * 8192)) return 1;
     if (bf) {
         if (dev_alloc(c, &ws.win_norm_b, F * 128)) return 1;
-        if (!c->chk_raw.empty() && (dev_alloc(c, &ws.z0b, Wn * 12 * 256) || dev_alloc(c, &ws.z1b, Wn * 48 * 128) ||
-                                    dev_alloc(c, &ws.z2b, Wn * 192 * 64) || dev_alloc(c, &ws.zyb, Wn * 192 * 64))) return 1;
-        if (c->chunker_tc) {
-            if (dev_alloc(c, &ws.cinb, Wn * 12 * 384) || dev_alloc(c, &ws.z3b, Wn * 192 * 64 + 512)) return 1;
+        if (!c->chk_raw.empty()) {
+            if (dev_alloc(c, &ws.z0b, Wn * 12 * 256) || dev_alloc(c, &ws.z1b, Wn * 48 * 128) || dev_alloc(c, &ws.z2b, Wn * 192 * 64) ||
+                dev_alloc(c, &ws.zyb, Wn * 192 * 64) || dev_alloc(c, &ws.cinb, Wn * 12 * 384) || dev_alloc(c, &ws.z3b, Wn * 192 * 64 + 512)) return 1;
             CUtensorMap *ta = new CUtensorMap(), *tb = new CUtensorMap();
             c->c_post_tmA = ta; c->c_post_tmB = tb;
             if (make_tma_2d_bf16(ta, ws.z3b, (long long)Wn * 8, 512, 24 * 64, 128) || make_tma_2d_bf16(tb, c->c_post_wbf, 256, 512, 512, 128)) return 1;
@@ -327,8 +324,10 @@ static int finalize(b2_ctx *c) {
     }
     if (dev_alloc(c, &ws.audio, F * 256)) return 1;
     if (!c->chk_raw.empty()) {
-        if (dev_alloc(c, &ws.z0, Wn * 12 * 192) || dev_alloc(c, &ws.z1, Wn * 48 * 128) || dev_alloc(c, &ws.z2, Wn * 192 * 64) ||
-            dev_alloc(c, &ws.zy, Wn * 192 * 64) || dev_alloc(c, &ws.z3, Wn * 192 * 64) || dev_alloc(c, &ws.post, Wn * 2048)) return 1;
+        if (bf) {
+            if (dev_alloc(c, &ws.z2, Wn * 192 * 64) || dev_alloc(c, &ws.post, Wn * 2048)) return 1;
+        } else if (dev_alloc(c, &ws.z0, Wn * 12 * 192) || dev_alloc(c, &ws.z1, Wn * 48 * 128) || dev_alloc(c, &ws.z2, Wn * 192 * 64) ||
+                   dev_alloc(c, &ws.zy, Wn * 192 * 64) || dev_alloc(c, &ws.z3, Wn * 192 * 64) || dev_alloc(c, &ws.post, Wn * 2048)) return 1;
     }
     if (dev_alloc(c, &ws.audio16k, Wn * 2048)) return 1;
     if (c->has_postnet) {
@@ -421,18 +420,13 @@ static int vocoder_bf16(b2_ctx *c, const float *xn, int W, int T, float *audio, 
     }
     const __nv_bfloat16 *stage_in = ws.c0b;
     int Tc = T;
-    bool post_done = false;
     for (int i = 0; i < 4; i++) {
-        // One launch per ResBlock where the fused kernel covers the stage (conv_resblock.cu); B2_RESBLOCK_FUSION=0 keeps the
-        // conv-by-conv path everywhere.
-        static const bool fusion_on = !(getenv("B2_RESBLOCK_FUSION") && atoi(getenv("B2_RESBLOCK_FUSION")) == 0);
-        static const bool post_fusion = !(getenv("B2_POST_FUSION") && atoi(getenv("B2_POST_FUSION")) == 0);
-        const bool fused = fusion_on && c->rb[i][0].tmap && c->rb[i][1].tmap && c->rb[i][2].tmap;
+        // One launch per ResBlock where the fused kernel covers the stage (conv_resblock.cu: C = 128, 64, 32); stage 0 runs conv by conv.
+        const bool fused = c->rb[i][0].tmap && c->rb[i][1].tmap && c->rb[i][2].tmap;
         // Stage 3: the stacked-output ResBlock kernel computes the stage's upsampler itself (conv_resblock_t.cu, UP): no upsampler launch, and
-        // x (1.6 GB of fp32 at 4,096 windows, read by three launches) never exists in HBM.  Needs all three ResBlocks on that kernel; off with
-        // B2_UP_FUSION=0, with B2_RB_T=0, and while the stage-boundary taps are being recorded (they want x).
-        static const bool up_fusion_on = !(getenv("B2_UP_FUSION") && atoi(getenv("B2_UP_FUSION")) == 0);
-        const bool up_fused = fused && up_fusion_on && i == 3 && resblock_t_enabled() && c->up[i].tmap_q && !c->taps[1 + 2 * i] &&
+        // x (1.6 GB of fp32 at 4,096 windows, read by three launches) never exists in HBM.  Needs all three ResBlocks on that kernel; not while
+        // the stage-boundary taps are being recorded (they want x).
+        const bool up_fused = fused && i == 3 && c->up[i].tmap_q && !c->taps[1 + 2 * i] &&
                               c->rb[i][0].tmap_t && c->rb[i][1].tmap_t && c->rb[i][2].tmap_t;
         if (!up_fused) {
             UmmaConvArgs u;
@@ -452,8 +446,7 @@ static int vocoder_bf16(b2_ctx *c, const float *xn, int W, int T, float *audio, 
                 else {
                     ra.div = 3.0f;
                     if (i < 3) ra.outb = ws.sb;
-                    else if (post_fusion) { ra.post_w = c->post_w; ra.post_b = c->post_b; ra.audio = audio; post_done = true; }   // conv_post + tanh in the same launch
-                    else ra.out32 = ws.s0;
+                    else { ra.post_w = c->post_w; ra.post_b = c->post_b; ra.audio = audio; }   // conv_post + tanh in the same launch
                 }
                 PROF(PC_RESBLOCK, launch_resblock(ra, st));
             }
@@ -466,17 +459,13 @@ static int vocoder_bf16(b2_ctx *c, const float *xn, int W, int T, float *audio, 
                 const __nv_bfloat16 *xb = (d == 0) ? ws.hb : ws.rb;
                 const bool last = d == 2;
                 // epilogue of the pair: next pair's residual + operand, or the MRF mean (modeling_speecht5.py:3069-3072):
-                // s0 = x0; s0 += x1; (s0 + x2) / 3
+                // s0 = x0; s0 += x1; (s0 + x2) / 3 as the operand of the next upsampler
                 float *o32 = nullptr; __nv_bfloat16 *ob = nullptr; const float *accs = nullptr; float dv = 1.0f;
                 if (!last) { o32 = ws.r; ob = ws.rb; }
                 else {
                     accs = (j > 0) ? ws.s0 : nullptr;
                     if (j < 2) o32 = ws.s0;
-                    else {
-                        dv = 3.0f;
-                        if (i < 3) ob = ws.sb;      // operand of the next upsampler
-                        else o32 = ws.s0;           // fp32 input of conv_post
-                    }
+                    else { dv = 3.0f; ob = ws.sb; }
                 }
                 UmmaConvArgs u1;
                 u1.in = xb; u1.layer = &c->res1[i][j][d]; u1.outb = ws.yb; u1.outb_slope = 0.1f; u1.W = W; u1.T = Tc;
@@ -489,7 +478,6 @@ static int vocoder_bf16(b2_ctx *c, const float *xn, int W, int T, float *audio, 
         }
         stage_in = ws.sb;
     }
-    if (!post_done) PROF(PC_CONV_POST, launch_conv_post(ws.s0, c->post_w, c->post_b, audio, W, Tc, st));
     return 0;
 }
 
@@ -502,16 +490,12 @@ static int chunker_fwd(b2_ctx *c, const float *win_raw, const float *audio, int 
     Workspace &ws = c->ws;
     if (!c->cwm) return set_error("chunker weights were not loaded into this context");
     if (c->mode == B2_MODE_BF16) {
-        // middle of the chunker on tensor cores (bf16 operands, fp32 accumulate, fp32 residual): 2 upsamplers + the ResBlock
+        // the whole chunker on tensor cores (bf16 operands, fp32 accumulate, fp32 residual): the prologue, 2 upsamplers, the ResBlock, post_conv
+        PROF(PC_OTHER, launch_chunker_in(win_raw, audio, ws.cinb, W, st));
         UmmaConvArgs u;
-        if (c->chunker_tc) {
-            PROF(PC_OTHER, launch_chunker_in(win_raw, audio, ws.cinb, W, st));
-            u.in = ws.cinb; u.layer = &c->c_pre_tc; u.outb = ws.z0b; u.outb_slope = 0.01f; u.W = W; u.T = 12;
-            PROF(PC_CONV_TC, launch_conv_umma(u, st));
-            u = UmmaConvArgs();
-        } else {
-            PROF(PC_OTHER, launch_chunker_pre(win_raw, audio, c->cwm, c->cbm, c->cwa, c->cba, nullptr, ws.z0b, W, st));
-        }
+        u.in = ws.cinb; u.layer = &c->c_pre_tc; u.outb = ws.z0b; u.outb_slope = 0.01f; u.W = W; u.T = 12;
+        PROF(PC_CONV_TC, launch_conv_umma(u, st));
+        u = UmmaConvArgs();
         u.in = ws.z0b; u.layer = &c->c_up[0]; u.outb = ws.z1b; u.outb_slope = 0.01f; u.W = W; u.T = 12;
         PROF(PC_CONV_TC, launch_conv_umma(u, st));
         u = UmmaConvArgs();
@@ -521,31 +505,26 @@ static int chunker_fwd(b2_ctx *c, const float *win_raw, const float *audio, int 
         u.in = ws.z2b; u.layer = &c->c_res1; u.outb = ws.zyb; u.outb_slope = 0.01f; u.W = W; u.T = 192;
         PROF(PC_CONV_TC, launch_conv_umma(u, st));
         u = UmmaConvArgs();
-        u.in = ws.zyb; u.layer = &c->c_res2; u.residual = ws.z2; u.W = W; u.T = 192;
-        if (c->chunker_tc) { u.outb = ws.z3b; u.outb_slope = 0.01f; } else u.out32 = ws.z3;
+        u.in = ws.zyb; u.layer = &c->c_res2; u.residual = ws.z2; u.outb = ws.z3b; u.outb_slope = 0.01f; u.W = W; u.T = 192;
         PROF(PC_CONV_TC, launch_conv_umma(u, st));
-        if (c->chunker_tc) {
-            // post_conv (64 -> 256, k8, stride 24, no padding; HelloSippyRT.py:233-234) = [W*8][512] x [512][256]
-            GemmTcArgs g;
-            g.tmA = reinterpret_cast<const CUtensorMap *>(c->c_post_tmA); g.tmB = reinterpret_cast<const CUtensorMap *>(c->c_post_tmB);
-            g.bias = c->c_post.bias; g.out32 = ws.post; g.M = W * 8; g.N = 256; g.K = 512; g.nt = 128; g.pdl = pdl_enabled();
-            PROF(PC_CONV_TC, launch_gemm_tc(g, st));
-            PROF(PC_OTHER, launch_chunker_final(audio, ws.post, out, W, st));
-            return 0;
-        }
-    } else {
-    PROF(PC_OTHER, launch_chunker_pre(win_raw, audio, c->cwm, c->cbm, c->cwa, c->cba, ws.z0, nullptr, W, st));
-    ConvArgs a0 = conv_args(c->c_up[0], ws.z0, ws.z1, W, 12, 12, 0.01f);
-    PROF(PC_CONV_F32, launch_conv_simt(a0, st));
-    a0 = conv_args(c->c_up[1], ws.z1, ws.z2, W, 48, 48, 0.01f);
-    PROF(PC_CONV_F32, launch_conv_simt(a0, st));
-    a0 = conv_args(c->c_res1, ws.z2, ws.zy, W, 192, 192, 0.01f);
-    PROF(PC_CONV_F32, launch_conv_simt(a0, st));
-    a0 = conv_args(c->c_res2, ws.zy, ws.z3, W, 192, 192, 0.01f);
-    a0.residual = ws.z2;
-    PROF(PC_CONV_F32, launch_conv_simt(a0, st));
+        // post_conv (64 -> 256, k8, stride 24, no padding; HelloSippyRT.py:233-234) = [W*8][512] x [512][256]
+        GemmTcArgs g;
+        g.tmA = reinterpret_cast<const CUtensorMap *>(c->c_post_tmA); g.tmB = reinterpret_cast<const CUtensorMap *>(c->c_post_tmB);
+        g.bias = c->c_post.bias; g.out32 = ws.post; g.M = W * 8; g.N = 256; g.K = 512; g.nt = 128; g.pdl = pdl_enabled();
+        PROF(PC_CONV_TC, launch_gemm_tc(g, st));
+        PROF(PC_OTHER, launch_chunker_final(audio, ws.post, out, W, st));
+        return 0;
     }
-    ConvArgs a;
+    PROF(PC_OTHER, launch_chunker_pre(win_raw, audio, c->cwm, c->cbm, c->cwa, c->cba, ws.z0, W, st));
+    ConvArgs a = conv_args(c->c_up[0], ws.z0, ws.z1, W, 12, 12, 0.01f);
+    PROF(PC_CONV_F32, launch_conv_simt(a, st));
+    a = conv_args(c->c_up[1], ws.z1, ws.z2, W, 48, 48, 0.01f);
+    PROF(PC_CONV_F32, launch_conv_simt(a, st));
+    a = conv_args(c->c_res1, ws.z2, ws.zy, W, 192, 192, 0.01f);
+    PROF(PC_CONV_F32, launch_conv_simt(a, st));
+    a = conv_args(c->c_res2, ws.zy, ws.z3, W, 192, 192, 0.01f);
+    a.residual = ws.z2;
+    PROF(PC_CONV_F32, launch_conv_simt(a, st));
     a = conv_args(c->c_post, ws.z3, ws.post, W, 192, 8, 0.01f);
     PROF(PC_CONV_F32, launch_conv_simt(a, st));
     PROF(PC_OTHER, launch_chunker_final(audio, ws.post, out, W, st));

@@ -15,20 +15,11 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 // try_wait carries a suspend-time hint: without one the hardware's default time limit is a few tens of cycles, and the waiting warps (TMA producer,
 // MMA issuers, epilogue warps between sub-tiles) re-issue the try_wait + branch pair all the time -- in k_resblock<32> a quarter of all executed
 // warp instructions were this polling (ncu source page, round 2), on the same schedulers the epilogue math needs.  With the hint the warp is parked
-// until the phase completes (or the limit passes).  -DB2_MBAR_NO_HINT builds the old loop for A/B runs.
+// until the phase completes (or the limit passes).
 #ifndef B2_MBAR_HINT_NS
 #define B2_MBAR_HINT_NS 0x989680
 #endif
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-#ifdef B2_MBAR_NO_HINT
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n\t"
-        "@P1 bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t}" ::"r"(bar), "r"(parity) : "memory");
-#else
     asm volatile(
         "{\n\t.reg .pred P1;\n\t"
         "WAIT_%=:\n\t"
@@ -36,7 +27,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
         "@P1 bra DONE_%=;\n\t"
         "bra WAIT_%=;\n\t"
         "DONE_%=:\n\t}" ::"r"(bar), "r"(parity), "r"((uint32_t)B2_MBAR_HINT_NS) : "memory");
-#endif
 }
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
@@ -44,14 +34,6 @@ __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
 __device__ __forceinline__ void tma_load_3d(uint32_t dst, const void *tmap, uint32_t bar, int c0, int c1, int c2) {
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
                  ::"r"(dst), "l"(tmap), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-// the same load delivered to the same shared-memory offset (and signalled on the same mbarrier offset) of every CTA in cta_mask
-__device__ __forceinline__ void tma_load_3d_mc(uint32_t dst, const void *tmap, uint32_t bar, int c0, int c1, int c2, uint16_t cta_mask) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;"
-                 ::"r"(dst), "l"(tmap), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(cta_mask) : "memory");
 }
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {

@@ -67,7 +67,8 @@ SHAPES = [
 def _stacked_kernel_for_every_tap_count():
     """C = 32 shapes go to the stacked-output kernel (conv_resblock_t.cu) from five taps up by default; in this module also the three-tap
     shapes do, so that both of its MMA issue paths (unrolled k = 3 / 7 / 11, table-driven otherwise) are checked against torch.  The
-    time-as-M kernel's C = 32 path is covered by test_time_as_m_kernel_c32 below and by tests/test_gpu_kernel_variants.py."""
+    time-as-M kernel's C = 32 path is covered by test_time_as_m_kernel_c32 below and, inside the bf16 tail, by the stage-boundary taps
+    test of tests/test_gpu_tail.py."""
     from infernos_b200 import _lib
     lib = _lib.load()
     lib.b2_debug_set_stacked_min_taps(3)

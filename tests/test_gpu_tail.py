@@ -93,6 +93,19 @@ def test_vocoder_bf16_tracks_its_cpu_emulation(tail16, sds):
     assert snr(emu, got) >= 42.0
 
 
+def test_vocoder_bf16_with_taps_matches_vocoder(tail16):
+    """Recording the stage-boundary taps runs stage 3 differently: its upsampler is a launch of its own (the fused path never writes
+    x to memory), and the k = 3 ResBlock then runs on the time-as-M kernel.  Only this path reaches them in bf16 mode.  The operands
+    are rounded at the same points as in vocoder(); only the fp32 summation order differs."""
+    mel = synth.synth_mel(8, 12, seed=314).cuda()
+    ref = tail16.vocoder(mel).cpu()
+    got, taps = tail16.vocoder_with_taps(mel, names=("up3",))
+    assert taps["up3"].shape == (8, 32, 12 * 256)
+    s = snr(ref, got.cpu())
+    print("bf16 vocoder with taps vs without: %.1f dB" % s)
+    assert s > 46.0
+
+
 def _replay(tail, law=0):
     """Replays the scripted run of the REAL infer()/unbatch_and_dispatch() (tests/golden/infer_golden.npz)."""
     from oracle import tail as otail

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Timing of the fused resample+encode kernel at several row lengths (B2_RS_BLOCKS = resident CTAs per SM)."""
+"""Timing of the fused resample+encode kernel at several row lengths."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -16,7 +16,7 @@ for rows, L in ((100_000, 320), (100_000, 1600), (20_000, 8192), (4096, 8192), (
     x = (torch.rand(rows, L, device="cuda") * 2 - 1) * 0.9
     ms = timed(lambda: engine.resample_g711_encode(x))
     nb = 9.0 * rows * (L // 2)
-    print(os.environ.get("B2_RS_BLOCKS", "2"), rows, L, round(ms, 4), "ms", round(nb / ms / 1e6), "GB/s", round(nb / ms / 1e6 / 6446.6, 3))
+    print(rows, L, round(ms, 4), "ms", round(nb / ms / 1e6), "GB/s", round(nb / ms / 1e6 / 6446.6, 3))
 
 # 8k -> 16k side (G711Codec.decode + AudioChunk.resample): 0.5 B in + 4 B out per 16 kHz output sample
 for rows, L in ((100_000, 160), (100_000, 800), (20_000, 4096)):
