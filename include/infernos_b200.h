@@ -218,6 +218,58 @@ B2_API int b2_enc_forward(b2_enc *enc, const int32_t *d_ids, const int32_t *h_le
 /* token ids outside [0, 81) are embedded as zeros and flagged; reported here (stream synchronised) or by the next call */
 B2_API int b2_enc_poll_errors(b2_enc *enc, void *stream);
 
+/* ---- sentence server: token ids in, G.711 chunks out ---------------------------------------------------------------------------------
+ * Replaces the reference's worker loop  infer() -> unbatch_and_dispatch()  (Cluster/InfernTTSWorker.py:83-92) together with the engine call it
+ * drives (HelloSippyTTSRT/HelloSippyRTPipe.py:195-259), for whole sentences.  A native driver thread runs engine calls back to back; each call
+ *   admits pending sentences into free slots (one encoder pass + b2_dec_start for all of them), runs ONE b2_dec_steps(16) over every live
+ *   slot whatever call admitted it, applies the reference's stop rule on the device (:225-228), runs the fused tail with the post-net
+ *   (b2_tts_tail2, B2_TAIL_APPLY_POSTNET) and copies the bytes and the per-sentence slice [startoff, endoff) to pinned host memory,
+ * with no host synchronisation between those parts and `depth` calls in flight.  A completer thread turns each finished call into records and
+ * returns the slots of ended sentences to the pool.  Semantics are HelloSippyRTPipe's: 16 decoder steps = 32 frames = 4,096 bytes per sentence
+ * and call, starts_at = 1, a sentence ends 2 steps after the stop fires, minlen / maxlen from the padded token length of the sentence's
+ * admission round (maxlen capped at max_steps - 20), prenet dropout masks drawn on the device from (seed, decoder call counter).
+ * The server owns ctx, enc and dec while it exists: do not call other b2_* entry points on them concurrently, and destroy it first. */
+typedef struct b2_tts_server b2_tts_server;
+typedef struct b2_tts_chunk {
+    uint64_t tag;            /* the caller's tag */
+    int64_t call;            /* engine call that produced this record (0, 1, ...) */
+    int64_t admit_call;      /* engine call at which the sentence was admitted */
+    int64_t t_submit_ns;     /* CLOCK_MONOTONIC: entry into b2_tts_server_submit */
+    int64_t t_done_ns;       /* CLOCK_MONOTONIC: the call's bytes were in pinned host memory */
+    int64_t g711_offset;     /* offset of this record's nbytes in the h_g711 buffer given to b2_tts_server_poll (-1 if none was given) */
+    int32_t nbytes;          /* G.711 bytes of this sentence in this call (may be 0 on the ended record) */
+    int32_t ended;           /* 1: the sentence's last record; nothing follows it */
+} b2_tts_chunk;
+typedef struct b2_tts_server_stats {
+    uint64_t calls;          /* engine calls completed */
+    uint64_t submitted, admitted, ended;
+    uint64_t admission_rounds;
+    uint64_t rows;           /* sum over calls of the rows handed to the decoder (live + retired) */
+    uint64_t live_rows;      /* sum over calls of the rows that were still live on the device */
+    uint64_t padded_rows;    /* scratch sessions added to tail launches to reach a graph bucket */
+    uint64_t graph_launches, graphs_built, max_rows;
+    uint64_t capacity;       /* sentences in flight at most (slots) */
+    uint64_t depth;
+} b2_tts_server_stats;
+/* ctx needs post-net weights; law B2_LAW_ULAW / ALAW; depth: engine calls in flight (1..4); use_graphs: each call's tail is one CUDA graph
+ * launch (rows padded to a bucket with the scratch session).  Reference defaults: threshold 0.5, minlenratio 0, maxlenratio 20. */
+B2_API b2_tts_server *b2_tts_server_create(b2_ctx *ctx, b2_enc *enc, b2_dec *dec, int law, int depth, int use_graphs, float threshold,
+                                           float minlenratio, float maxlenratio, uint64_t seed);
+/* stops the threads (work in flight is abandoned), waits for the device and frees the server; ctx, enc and dec stay valid */
+B2_API void b2_tts_server_destroy(b2_tts_server *s);
+/* n sentences: h_lens[n] token counts, h_ids[sum(h_lens)] int32 host token ids in [0, vocab) back to back, h_speakers (n, 512) fp32 host
+ * (normalised on the device as b2_dec_start does), tags[n] the caller's ids.  Rejected with nothing enqueued: NULL pointers, a sentence of
+ * no token, more tokens than the encoder's max_len / max_tokens or the decoder's max_enc_len, a token id outside the vocabulary.  Blocks
+ * while every slot is taken by a sentence that has not ended (back-pressure) and fails after 20 s of that.  Sentences enqueued together
+ * (all of them when the slots allow) are admitted in one round. */
+B2_API int b2_tts_server_submit(b2_tts_server *s, const int32_t *h_ids, const int32_t *h_lens, int n, const float *h_speakers, const uint64_t *tags);
+/* up to max_out records, oldest call first; their bytes are copied to h_g711 (may be NULL) at out[i].g711_offset (a record whose bytes
+ * do not fit waits for the next poll).  timeout_ms: 0 = do not wait, < 0 = wait.  Returns the count, or a negative value on error. */
+B2_API int b2_tts_server_poll(b2_tts_server *s, b2_tts_chunk *out, int max_out, uint8_t *h_g711, size_t g711_capacity, int timeout_ms);
+/* returns when every sentence submitted so far has ended (its records may still be waiting for b2_tts_server_poll) */
+B2_API int b2_tts_server_flush(b2_tts_server *s, int timeout_ms);
+B2_API int b2_tts_server_get_stats(b2_tts_server *s, b2_tts_server_stats *out);
+
 /* ---- Core/Codecs (G711.py:25-47), ctx-less, stateless ----------------------------------------------- */
 /* G711Codec.encode: clamp(x*32767,-32768,32767) -> int16 (trunc toward zero) -> G.711 code.  n samples. */
 B2_API int b2_g711_encode_f32(const float *d_in, size_t n, int law, uint8_t *d_out, void *stream);

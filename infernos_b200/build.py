@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libinfernos_b200.so")
-SOURCES = ["tail.cu", "codec_kernels.cu", "conv_simt.cu", "conv_umma.cu", "conv_resblock.cu", "conv_resblock_t.cu", "sched.cu", "decoder.cu", "encoder.cu"]
+SOURCES = ["tail.cu", "codec_kernels.cu", "conv_simt.cu", "conv_umma.cu", "conv_resblock.cu", "conv_resblock_t.cu", "sched.cu", "server.cu", "decoder.cu", "encoder.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
 

@@ -23,6 +23,7 @@
 #include "umma_ptx.cuh"
 #include "gemm_tc.cuh"
 #include "layers.cuh"
+#include "serve.cuh"
 #include "../../include/infernos_b200.h"
 
 #include <cuda.h>
@@ -760,6 +761,10 @@ int start_impl(b2_dec *d, const int32_t *d_slots, const float *d_enc, int n, int
         cudaError_t _e = cudaSetDevice((d)->device);                                                  \
         if (_e != cudaSuccess) return set_error("cudaSetDevice(%d): %s", (d)->device, cudaGetErrorString(_e)); \
     }
+
+void b2::dec_limits(const b2_dec *d, int *max_sessions, int *max_steps, int *max_enc_len) {
+    *max_sessions = d->max_sessions; *max_steps = d->max_steps; *max_enc_len = d->max_enc;
+}
 
 extern "C" {
 

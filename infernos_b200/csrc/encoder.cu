@@ -17,6 +17,7 @@
 // gemm_tc.cuh (bf16 operands by TMA, fp32 accumulators, bias / GELU in the epilogue); fp32 residual stream, LayerNorm, q / k / v and attention.
 #include "common.cuh"
 #include "layers.cuh"
+#include "serve.cuh"
 #include "../../include/infernos_b200.h"
 
 #include <math.h>
@@ -312,6 +313,10 @@ int pass_impl(b2_enc *d, const int32_t *d_ids, int L, int s0, int ns, int row0, 
 }
 
 }  // namespace
+
+void b2::enc_limits(const b2_enc *e, int *max_tokens, int *max_len, int *vocab) {
+    *max_tokens = e->max_tokens; *max_len = e->max_len; *vocab = VOCAB;
+}
 
 #define ENC_GUARD(d)                                                                                  \
     if (!(d)) return set_error("null encoder handle");                                                \

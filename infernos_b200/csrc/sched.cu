@@ -15,13 +15,10 @@
 // With `depth` sub-batches in flight the H2D of sub-batch n+1 and the D2H of n-1 overlap the compute of n; the compute of successive
 // sub-batches is serialised on one stream (they share the context's workspaces).  Sessions per sub-batch are padded up to a bucket
 // size with a scratch session (slot id max_sessions) so that a few dozen graphs cover every batch size.
-#include "common.cuh"
-#include "ctx.cuh"
+#include "serve.cuh"
 #include "../../include/infernos_b200.h"
 
-#include <time.h>
 #include <string.h>
-#include <algorithm>
 #include <condition_variable>
 #include <deque>
 #include <map>
@@ -32,18 +29,6 @@
 using namespace b2;
 
 namespace {
-
-inline int64_t now_ns() {
-    timespec ts;
-    clock_gettime(CLOCK_MONOTONIC, &ts);
-    return (int64_t)ts.tv_sec * 1000000000ll + ts.tv_nsec;
-}
-
-// sessions per sub-batch are rounded up to: multiples of 8 up to 64, of 32 up to 512, of 128 beyond (<= 12.5 % padding above 64)
-inline int bucket_of(int n, int cap) {
-    int b = n <= 64 ? ((n + 7) / 8) * 8 : n <= 512 ? ((n + 31) / 32) * 32 : ((n + 127) / 128) * 128;
-    return std::min(b, cap);
-}
 
 struct Batch {
     int id = 0;
@@ -100,21 +85,10 @@ int sched_fail(b2_sched *s, const char *what) {
 
 // captures the tail over `b`'s device staging buffers at a padded sub-batch size `nb` and instantiates it (nothing is launched)
 int build_graph(b2_sched *s, Batch *b, int nb) {
-    b2_ctx *c = s->ctx;
-    const bool pn = (s->flags & B2_TAIL_APPLY_POSTNET) != 0;
-    cudaGraph_t g = nullptr;
     cudaGraphExec_t ge = nullptr;
-    const uint64_t l0 = g_launches.load();
-    B2_CUDA_OK(cudaStreamBeginCapture(s->s_c, cudaStreamCaptureModeRelaxed)      /* relaxed: a kernel's first launch may set its function attributes */);
-    const int rc = tail_device(c, b->d_slots, b->d_mel, nb, s->nframes, s->law, pn, b->d_out, nullptr, s->s_c, false, true);
-    cudaError_t e = cudaStreamEndCapture(s->s_c, &g);
-    if (rc) { if (g) cudaGraphDestroy(g); return 1; }
-    if (e != cudaSuccess) return set_error("cudaStreamEndCapture: %s", cudaGetErrorString(e));
-    e = cudaGraphInstantiate(&ge, g, 0);
-    cudaGraphDestroy(g);
-    if (e != cudaSuccess) return set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e));
-    const int nk = (int)(g_launches.load() - l0);          // kernel nodes: counted by the launch wrappers while capturing
-    g_launches.fetch_sub((uint64_t)nk);                    // ... and only charged when the graph actually runs
+    int nk = 0;
+    if (capture_tail_graph(s->ctx, b->d_slots, b->d_mel, nb, s->nframes, s->law, (s->flags & B2_TAIL_APPLY_POSTNET) != 0, b->d_out, s->s_c, &ge, &nk))
+        return 1;
     b->graphs.emplace(nb, std::make_pair(ge, nk));
     s->n_graphs++;
     return 0;
@@ -225,6 +199,37 @@ void recycle(b2_sched *s, Batch *b) {      // under the mutex
 
 }  // namespace
 
+namespace b2 {
+
+int capture_tail_graph(b2_ctx *c, const int32_t *d_slots, const float *d_mel, int nb, int nframes, int law, bool apply_postnet, uint8_t *d_g711,
+                       cudaStream_t st, cudaGraphExec_t *exec, int *nk) {
+    cudaGraph_t g = nullptr;
+    cudaGraphExec_t ge = nullptr;
+    const uint64_t l0 = g_launches.load();
+    B2_CUDA_OK(cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed)      /* relaxed: a kernel's first launch may set its function attributes */);
+    const int rc = tail_device(c, d_slots, d_mel, nb, nframes, law, apply_postnet, d_g711, nullptr, st, false, true);
+    cudaError_t e = cudaStreamEndCapture(st, &g);
+    if (rc) { if (g) cudaGraphDestroy(g); return 1; }
+    if (e != cudaSuccess) return set_error("cudaStreamEndCapture: %s", cudaGetErrorString(e));
+    e = cudaGraphInstantiate(&ge, g, 0);
+    cudaGraphDestroy(g);
+    if (e != cudaSuccess) return set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e));
+    *nk = (int)(g_launches.load() - l0);                   // kernel nodes: counted by the launch wrappers while capturing
+    g_launches.fetch_sub((uint64_t)*nk);                   // ... and only charged when the graph actually runs
+    *exec = ge;
+    return 0;
+}
+
+int warm_tail(b2_ctx *c, int32_t *d_slots, const float *d_mel, int nb, int nframes, int law, bool apply_postnet, uint8_t *d_g711, cudaStream_t st) {
+    std::vector<int32_t> pad((size_t)nb, c->max_sessions);
+    B2_CUDA_OK(cudaMemcpyAsync(d_slots, pad.data(), (size_t)nb * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if (tail_device(c, d_slots, d_mel, nb, nframes, law, apply_postnet, d_g711, nullptr, st, false, true)) return 1;
+    B2_CUDA_OK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+}  // namespace b2
+
 extern "C" {
 
 b2_sched *b2_sched_create(b2_ctx *c, int nframes, int law, int flags, int max_batch, int depth, int use_graphs) {
@@ -272,15 +277,9 @@ b2_sched *b2_sched_create(b2_ctx *c, int nframes, int law, int flags, int max_ba
         b2_sched_destroy(s);
         return nullptr;
     }
-    // one eager pass over scratch sessions only: every kernel of the path sets its attributes before anything is captured
-    {
-        Batch *b = s->pool[0];
-        const int nb = std::min(8, max_batch);
-        for (int i = 0; i < nb; i++) b->h_slots[i] = c->max_sessions;
-        bool w = cudaMemcpyAsync(b->d_slots, b->h_slots, (size_t)nb * sizeof(int32_t), cudaMemcpyHostToDevice, s->s_c) == cudaSuccess;
-        w = w && !tail_device(c, b->d_slots, b->d_mel, nb, nframes, law, (flags & B2_TAIL_APPLY_POSTNET) != 0, b->d_out, nullptr, s->s_c, false, true);
-        w = w && cudaStreamSynchronize(s->s_c) == cudaSuccess;
-        if (!w) { b2_sched_destroy(s); return nullptr; }
+    if (warm_tail(c, s->pool[0]->d_slots, s->pool[0]->d_mel, std::min(8, max_batch), nframes, law, (flags & B2_TAIL_APPLY_POSTNET) != 0, s->pool[0]->d_out, s->s_c)) {
+        b2_sched_destroy(s);
+        return nullptr;
     }
     s->open = s->pool[0];
     for (int i = 1; i < nbuf; i++) s->free_q.push_back(s->pool[i]);

@@ -524,6 +524,135 @@ class TTSEncoder:
             _lib.check(self.lib.b2_enc_poll_errors(self.h, _stream_ptr(self.device)), "enc_poll_errors")
 
 
+class _TTSChunk(ctypes.Structure):
+    _fields_ = [("tag", ctypes.c_uint64), ("call", ctypes.c_int64), ("admit_call", ctypes.c_int64), ("t_submit_ns", ctypes.c_int64),
+                ("t_done_ns", ctypes.c_int64), ("g711_offset", ctypes.c_int64), ("nbytes", ctypes.c_int32), ("ended", ctypes.c_int32)]
+
+
+class _TTSServerStats(ctypes.Structure):
+    _fields_ = [(k, ctypes.c_uint64) for k in ("calls", "submitted", "admitted", "ended", "admission_rounds", "rows", "live_rows", "padded_rows",
+                                               "graph_launches", "graphs_built", "max_rows", "capacity", "depth")]
+
+
+class TTSServer:
+    """Whole sentences in, G.711 chunks out (b2_tts_server_*): the reference's worker loop around infer() / unbatch_and_dispatch()
+    (Cluster/InfernTTSWorker.py:83-92, HelloSippyRTPipe.py:195-259) as a native loop.  Every engine call admits the sentences submitted since
+    the last one, runs 16 decoder steps over every live sentence whatever call admitted it, applies the stop rule on the GPU and runs the tail
+    with the post-net; `depth` calls are in flight.  `tail` must hold post-net weights.  While the server exists it owns the tail, encoder
+    and decoder handles: do not call them, and close the server before them (closing the tail closes it)."""
+
+    def __init__(self, tail: "TTSTail", encoder: "TTSEncoder", decoder: "TTSDecoder", law: int = LAW_ULAW, depth: int = 2, threshold: float = 0.5,
+                 minlenratio: float = 0.0, maxlenratio: float = 20.0, seed: int = 0, use_graphs: bool = True, poll_capacity: int = 4096):
+        if law not in (LAW_ULAW, LAW_ALAW):
+            raise RuntimeError(f"law must be LAW_ULAW or LAW_ALAW, got {law!r}")
+        if not 1 <= int(depth) <= 4:
+            raise RuntimeError(f"depth must be 1..4, got {depth!r}")
+        if not tail.has_postnet:
+            raise RuntimeError("TTSServer needs a TTSTail built with post-net weights (postnet_sd)")
+        if not (minlenratio >= 0.0 and maxlenratio >= 0.0 and threshold == threshold):
+            raise RuntimeError("threshold must be a number and minlenratio / maxlenratio >= 0")
+        if int(poll_capacity) < 1:
+            raise RuntimeError("poll_capacity must be >= 1")
+        self.tail, self.encoder, self.decoder, self.lib = tail, encoder, decoder, tail.lib
+        with torch.cuda.device(tail.index):
+            self.h = self.lib.b2_tts_server_create(tail.ctx, encoder.h, decoder.h, int(law), int(depth), 1 if use_graphs else 0, float(threshold),
+                                                   float(minlenratio), float(maxlenratio), int(seed) & (2 ** 64 - 1))
+        if not self.h:
+            raise RuntimeError("b2_tts_server_create: " + self.lib.b2_last_error(None).decode())
+        if not hasattr(tail, "_schedulers"):
+            tail._schedulers = []
+        tail._schedulers.append(self)
+        self._cap = int(poll_capacity)
+        self._recs = (_TTSChunk * self._cap)()
+        self._bytes = torch.empty(self._cap * 4096, dtype=torch.uint8)
+
+    def close(self) -> None:
+        """Stops the loop (work in flight is dropped) and frees the server; the tail, encoder and decoder stay usable."""
+        if getattr(self, "h", None):
+            self.lib.b2_tts_server_destroy(self.h)
+            self.h = None
+            if self in getattr(self.tail, "_schedulers", []):
+                self.tail._schedulers.remove(self)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _handle(self):
+        if not getattr(self, "h", None):
+            raise RuntimeError("the TTSServer is closed")
+        return self.h
+
+    def submit(self, ids, speaker, tag: int) -> None:
+        """One sentence: ids = token ids (a 1-D sequence or tensor of ints), speaker = (512,) or (1, 512) x-vector (normalised on the GPU),
+        tag = the caller's unsigned 64-bit id, echoed in every record.  Blocks while every slot is busy."""
+        self.submit_many([ids], [speaker], [tag])
+
+    def submit_many(self, ids_list, speakers, tags) -> None:
+        """Several sentences at once (lists of what submit() takes); when the slots allow, they are admitted in one round.  Nothing is
+        enqueued if any of them is rejected."""
+        if not (len(ids_list) == len(speakers) == len(tags)):
+            raise RuntimeError("ids_list, speakers and tags must have the same length")
+        n = len(ids_list)
+        if n == 0:
+            return
+        toks, lens = [], []
+        for ids in ids_list:
+            t = torch.as_tensor(ids)
+            if t.dim() == 2 and t.size(0) == 1:
+                t = t[0]
+            if t.numel() < 1:
+                raise RuntimeError("a sentence needs at least one token")
+            if t.dim() != 1 or t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+                raise RuntimeError("ids must be a 1-D sequence of integer token ids")
+            if int(t.min()) < -2 ** 31 or int(t.max()) >= 2 ** 31:
+                raise RuntimeError("token ids must fit in int32")
+            toks.append(t.to("cpu", torch.int32))
+            lens.append(t.numel())
+        sp = []
+        for s in speakers:
+            v = torch.as_tensor(s).detach().to("cpu", torch.float32).reshape(-1)
+            if v.numel() != 512:
+                raise RuntimeError(f"a speaker vector must hold 512 values, got {v.numel()}")
+            sp.append(v)
+        tg = [int(t) for t in tags]
+        if any(not 0 <= t < 2 ** 64 for t in tg):
+            raise RuntimeError("tags must be unsigned 64-bit integers")
+        h = self._handle()
+        ids_t = torch.cat(toks).contiguous()
+        lens_t = torch.tensor(lens, dtype=torch.int32)
+        sp_t = torch.stack(sp).contiguous()
+        tags_a = (ctypes.c_uint64 * n)(*tg)
+        _lib.check(self.lib.b2_tts_server_submit(h, ids_t.data_ptr(), lens_t.data_ptr(), n, sp_t.data_ptr(), tags_a), "tts_server_submit")
+
+    def poll(self, timeout_ms: int = 0):
+        """-> list of (record, bytes): record a dict with tag, call, admit_call, nbytes, ended, t_submit_ns, t_done_ns; bytes the G.711
+        payload of that sentence in that call.  timeout_ms: 0 = do not wait, < 0 = wait for the next completed call."""
+        h = self._handle()
+        n = self.lib.b2_tts_server_poll(h, self._recs, self._cap, self._bytes.data_ptr(), self._bytes.numel(), int(timeout_ms))
+        if n < 0:
+            raise RuntimeError("infernos_b200 tts_server_poll: " + self.lib.b2_last_error(None).decode())
+        out = []
+        raw = self._bytes.numpy()
+        for r in self._recs[:n]:
+            rec = {k: int(getattr(r, k)) for k, _ in _TTSChunk._fields_ if k != "g711_offset"}
+            rec["ended"] = bool(rec["ended"])
+            out.append((rec, raw[r.g711_offset:r.g711_offset + r.nbytes].tobytes()))
+        return out
+
+    def flush(self, timeout_ms: int = 600000) -> None:
+        """Returns when every sentence submitted so far has ended (its records may still be waiting for poll)."""
+        h = self._handle()
+        _lib.check(self.lib.b2_tts_server_flush(h, int(timeout_ms)), "tts_server_flush")
+
+    def stats(self) -> dict:
+        h, st = self._handle(), _TTSServerStats()
+        _lib.check(self.lib.b2_tts_server_get_stats(h, ctypes.byref(st)), "tts_server_get_stats")
+        return {k: int(getattr(st, k)) for k, _ in _TTSServerStats._fields_}
+
+
 def postnet_layers(sd: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
     """Picks the post-net's conv / batch-norm tensors out of a SpeechT5 state_dict, whatever prefix they carry
     (`layers.0.conv.weight`, `speech_decoder_postnet.layers.0.conv.weight`, ...)."""
