@@ -228,17 +228,22 @@ B2_API int b2_enc_poll_errors(b2_enc *enc, void *stream);
  * returns the slots of ended sentences to the pool.  Semantics are HelloSippyRTPipe's: 16 decoder steps = 32 frames = 4,096 bytes per sentence
  * and call, starts_at = 1, a sentence ends 2 steps after the stop fires, minlen / maxlen from the padded token length of the sentence's
  * admission round (maxlen capped at max_steps - 20), prenet dropout masks drawn on the device from (seed, decoder call counter).
+ * Cancel (b2_tts_server_cancel, barge-in): a pending sentence leaves the queue at once and gets one record with call = admit_call = -1,
+ * nbytes = 0, ended = 2.  An admitted one is retired on the device at the start of the next engine call built: from that call on it takes no
+ * decoder step, and that call's record for it has nbytes = 0, ended = 2.  Records of calls built before the cancel (at most `depth`) still
+ * arrive with their bytes.  If one of those calls ends the sentence on its own, that record (ended = 1) stays its last one and the cancel
+ * does nothing: every sentence gets exactly one last record either way.
  * The server owns ctx, enc and dec while it exists: do not call other b2_* entry points on them concurrently, and destroy it first. */
 typedef struct b2_tts_server b2_tts_server;
 typedef struct b2_tts_chunk {
     uint64_t tag;            /* the caller's tag */
-    int64_t call;            /* engine call that produced this record (0, 1, ...) */
-    int64_t admit_call;      /* engine call at which the sentence was admitted */
+    int64_t call;            /* engine call that produced this record (0, 1, ...; -1: cancelled before admission) */
+    int64_t admit_call;      /* engine call at which the sentence was admitted (-1: never admitted) */
     int64_t t_submit_ns;     /* CLOCK_MONOTONIC: entry into b2_tts_server_submit */
     int64_t t_done_ns;       /* CLOCK_MONOTONIC: the call's bytes were in pinned host memory */
     int64_t g711_offset;     /* offset of this record's nbytes in the h_g711 buffer given to b2_tts_server_poll (-1 if none was given) */
     int32_t nbytes;          /* G.711 bytes of this sentence in this call (may be 0 on the ended record) */
-    int32_t ended;           /* 1: the sentence's last record; nothing follows it */
+    int32_t ended;           /* non-zero: the sentence's last record, nothing follows it; 2: ended by b2_tts_server_cancel */
 } b2_tts_chunk;
 typedef struct b2_tts_server_stats {
     uint64_t calls;          /* engine calls completed */
@@ -263,6 +268,11 @@ B2_API void b2_tts_server_destroy(b2_tts_server *s);
  * while every slot is taken by a sentence that has not ended (back-pressure) and fails after 20 s of that.  Sentences enqueued together
  * (all of them when the slots allow) are admitted in one round. */
 B2_API int b2_tts_server_submit(b2_tts_server *s, const int32_t *h_ids, const int32_t *h_lens, int n, const float *h_speakers, const uint64_t *tags);
+/* Cancels every sentence submitted with one of tags[0..n) whose last record has not been made yet.  Any thread; never waits for the GPU.
+ * Tags need not be unique: every matching sentence is cancelled.  Returns the number of sentences found (pending, or admitted and not yet
+ * known on the host to have ended); an unknown tag, a sentence that has ended and a second cancel of the same sentence count 0.  Negative
+ * on a NULL server, n < 0, tags == NULL with n > 0, or a stopped server. */
+B2_API int b2_tts_server_cancel(b2_tts_server *s, const uint64_t *tags, int n);
 /* up to max_out records, oldest call first; their bytes are copied to h_g711 (may be NULL) at out[i].g711_offset (a record whose bytes
  * do not fit waits for the next poll).  timeout_ms: 0 = do not wait, < 0 = wait.  Returns the count, or a negative value on error. */
 B2_API int b2_tts_server_poll(b2_tts_server *s, b2_tts_chunk *out, int max_out, uint8_t *h_g711, size_t g711_capacity, int timeout_ms);

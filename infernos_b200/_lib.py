@@ -50,6 +50,7 @@ SIGNATURES = {
     "b2_tts_server_create": (c_void_p, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_float, c_float, c_uint64]),
     "b2_tts_server_destroy": (None, [c_void_p]),
     "b2_tts_server_submit": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "b2_tts_server_cancel": (c_int, [c_void_p, c_void_p, c_int]),
     "b2_tts_server_poll": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_int]),
     "b2_tts_server_flush": (c_int, [c_void_p, c_int]),
     "b2_tts_server_get_stats": (c_int, [c_void_p, c_void_p]),

@@ -14,6 +14,12 @@
 // The host only learns that a sentence ended when its call completes.  With depth > 1 the next call has already been built with that
 // sentence in its row list, so k_tts_stop retires an ending row on the device (live[slot] = 0) and k_tts_rows of every later call turns the
 // row into the decoder's padding id -1 (the scratch slot: no step counted, nothing flagged) and the tail's scratch session.
+//
+// Cancellation (b2_tts_server_cancel) uses the same retirement.  A pending sentence is dropped from the queue on the host.  An admitted one
+// is queued as (slot, admission sequence number); the next build_call puts it into that call's cancel list if the slot still holds the same
+// admission, and k_tts_cancel clears live[slot] and marks the row, so k_tts_rows pads it and k_tts_stop reports {0, 0, 2}.  Whether the
+// sentence ended on its own in a call already in flight is known only on the device: there live[slot] is already 0 and the cancel does
+// nothing.  live goes from 1 to 0 once per admission, so every sentence gets exactly one last record.
 #include "serve.cuh"
 #include "../../include/infernos_b200.h"
 
@@ -68,15 +74,30 @@ __global__ void k_tts_rows(const int32_t *__restrict__ rows, int n, int nb, cons
     }
 }
 
+// cancels of this call: can[2i] = row, can[2i + 1] = slot.  A sentence still live on the device is retired and its row marked; one that a
+// call in flight already retired (a natural end) is left alone.  One thread per cancel.
+__global__ void k_tts_cancel(const int32_t *__restrict__ can, int n, int32_t *__restrict__ live, int32_t *__restrict__ mark) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int sl = can[2 * i + 1];
+    if (live[sl]) { live[sl] = 0; mark[can[2 * i]] = 1; }
+}
+
 // The stop rule of HelloSippyRTPipe._front_half (:417-421), step by step over this call's stop probabilities, then unbatch_prepare's slice
 // (:503-527): tri[i] = {startoff, endoff, ended} in bytes of this call's 4,096.  An ended sentence is retired (live = 0).  One thread per row.
+// mark (NULL when the call has no cancel): rows k_tts_cancel retired get {0, 0, 2}; the marks are cleared for the next call.
 __global__ void k_tts_stop(const int32_t *__restrict__ dslots, const float *__restrict__ prob, int n, float threshold, int32_t *__restrict__ idx,
                            int32_t *__restrict__ ends, const int32_t *__restrict__ minlen, const int32_t *__restrict__ maxlen, int32_t *__restrict__ live,
-                           int32_t *__restrict__ tri) {
+                           int32_t *__restrict__ mark, int32_t *__restrict__ tri) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int sl = dslots[i];
-    if (sl < 0) { tri[3 * i] = 0; tri[3 * i + 1] = 0; tri[3 * i + 2] = 0; return; }
+    if (sl < 0) {
+        int cancelled = 0;
+        if (mark) { cancelled = mark[i] ? 2 : 0; mark[i] = 0; }
+        tri[3 * i] = 0; tri[3 * i + 1] = 0; tri[3 * i + 2] = cancelled;
+        return;
+    }
     int t = idx[sl], e = ends[sl];
     const int lo = minlen[sl], hi = maxlen[sl];
     for (int s = 0; s < NSTEPS; s++) {
@@ -102,8 +123,10 @@ struct Pending {
 
 struct SlotInfo {
     uint64_t tag = 0;
+    uint64_t seq = 0;                          // admission sequence number: tells this sentence from a later one in the same slot
     int64_t t_submit = 0, admit_call = 0;
     bool live = false;
+    bool cancelled = false;                    // a cancel of this admission has been accepted
 };
 
 struct Done {                                  // the records of one completed call, waiting for poll()
@@ -115,13 +138,14 @@ struct Done {                                  // the records of one completed c
 // one engine call's pinned staging and device outputs; graphs bake this buffer's d_out in
 struct Call {
     int32_t *h_ids = nullptr, *h_len = nullptr, *h_adm = nullptr, *h_rows = nullptr, *h_tri = nullptr;
+    int32_t *h_can = nullptr;                  // cancel list: n_can (row, slot) pairs
     float *h_spk = nullptr;
     uint8_t *h_out = nullptr, *d_out = nullptr;
     int32_t *d_tri = nullptr;
     cudaEvent_t ev_c = nullptr, ev_out = nullptr;
     std::map<int, std::pair<cudaGraphExec_t, int>> graphs;    // bucket -> (instantiated tail graph, kernels in it)
     int64_t call = 0;
-    int n = 0, nb = 0, n_adm = 0, L = 0;
+    int n = 0, nb = 0, n_adm = 0, L = 0, n_can = 0;
     std::vector<int32_t> row_slot;
     std::vector<SlotInfo> row_info;            // the sentence each row belonged to when the call was built
 };
@@ -139,8 +163,9 @@ struct b2_tts_server {
     cudaStream_t s_c = nullptr, s_out = nullptr;
     // device state, indexed by slot
     int32_t *d_idx = nullptr, *d_ends = nullptr, *d_minlen = nullptr, *d_maxlen = nullptr, *d_live = nullptr;
-    // device workspaces shared by the calls (stream-ordered on s_c)
+    // device workspaces shared by the calls (stream-ordered on s_c); d_mark (by row) is all zero between calls
     int32_t *d_ids = nullptr, *d_len = nullptr, *d_adm = nullptr, *d_rows = nullptr, *d_dslots = nullptr, *d_tslots = nullptr;
+    int32_t *d_can = nullptr, *d_mark = nullptr;
     float *d_spk = nullptr, *d_enc = nullptr, *d_mel = nullptr, *d_prob = nullptr;
     std::vector<Call *> calls_pool;
     std::mutex mu;
@@ -149,9 +174,12 @@ struct b2_tts_server {
     std::vector<SlotInfo> slots;
     std::vector<int> free_slots;               // a stack: the lowest ids are handed out first
     std::vector<int> live_list;                // slots of admitted sentences not known to have ended, in admission order
+    std::vector<std::pair<int, uint64_t>> cancels;    // (slot, admission seq) accepted by cancel, for the next call built
+    std::vector<int> row_of;                   // by slot: row in the call being built (scratch of build_call)
     std::deque<Call *> free_q, inflight;
     std::deque<Done *> done_q;
     int64_t next_call = 0;
+    uint64_t next_seq = 0;
     int unfinished = 0;                        // submitted sentences whose ended record has not been made yet
     bool stop = false;
     std::string async_error;
@@ -185,12 +213,19 @@ int enqueue_call(b2_tts_server *s, Call *b) {
         k_tts_admit<<<na, 128, 0, st>>>(s->d_adm, na, s->d_idx, s->d_ends, s->d_minlen, s->d_maxlen, s->d_live, c->pre_pool);
         B2_LAUNCH_OK("k_tts_admit");
     }
+    const int nc = b->n_can;
+    if (nc > 0) {
+        B2_CUDA_OK(cudaMemcpyAsync(s->d_can, b->h_can, (size_t)2 * nc * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        k_tts_cancel<<<cdiv(nc, 128), 128, 0, st>>>(s->d_can, nc, s->d_live, s->d_mark);
+        B2_LAUNCH_OK("k_tts_cancel");
+    }
     const int nb = b->nb;
     B2_CUDA_OK(cudaMemcpyAsync(s->d_rows, b->h_rows, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     k_tts_rows<<<cdiv(nb, 128), 128, 0, st>>>(s->d_rows, n, nb, s->d_live, c->max_sessions, s->d_dslots, s->d_tslots);
     B2_LAUNCH_OK("k_tts_rows");
     if (b2_dec_steps(s->dec, s->d_dslots, n, NSTEPS, nullptr, s->seed, s->d_mel, s->d_prob, st)) return 1;
-    k_tts_stop<<<cdiv(n, 128), 128, 0, st>>>(s->d_dslots, s->d_prob, n, s->threshold, s->d_idx, s->d_ends, s->d_minlen, s->d_maxlen, s->d_live, b->d_tri);
+    k_tts_stop<<<cdiv(n, 128), 128, 0, st>>>(s->d_dslots, s->d_prob, n, s->threshold, s->d_idx, s->d_ends, s->d_minlen, s->d_maxlen, s->d_live,
+                                             nc > 0 ? s->d_mark : nullptr, b->d_tri);
     B2_LAUNCH_OK("k_tts_stop");
     if (s->use_graphs && !c->prof.on) {
         auto it = b->graphs.find(nb);
@@ -247,6 +282,7 @@ bool build_call(b2_tts_server *s, Call *b) {
         b->h_adm[i] = sl; b->h_adm[na + i] = minlen; b->h_adm[2 * na + i] = maxlen;
         SlotInfo &si = s->slots[(size_t)sl];
         si.tag = p.tag; si.t_submit = p.t_submit; si.admit_call = call; si.live = true;
+        si.seq = s->next_seq++; si.cancelled = false;
         s->live_list.push_back(sl);
         s->pending.pop_front();
     }
@@ -259,6 +295,20 @@ bool build_call(b2_tts_server *s, Call *b) {
         b->h_rows[i] = s->live_list[(size_t)i];
         b->row_info[(size_t)i] = s->slots[(size_t)s->live_list[(size_t)i]];
     }
+    // every accepted cancel enters this call, if its slot still holds the admission it was accepted for: the completer may have freed the
+    // slot on a natural end since, and this round may have given it to a newcomer
+    int nc = 0;
+    if (!s->cancels.empty()) {
+        for (int i = 0; i < n; i++) s->row_of[(size_t)s->live_list[(size_t)i]] = i;
+        for (const auto &q : s->cancels) {
+            const SlotInfo &si = s->slots[(size_t)q.first];
+            if (!si.live || si.seq != q.second) continue;
+            b->h_can[2 * nc] = s->row_of[(size_t)q.first]; b->h_can[2 * nc + 1] = q.first;
+            nc++;
+        }
+        s->cancels.clear();
+    }
+    b->n_can = nc;
     s->next_call++;
     if (na) { s->st.admission_rounds++; s->st.admitted += (uint64_t)na; }
     s->st.rows += (uint64_t)n; s->st.padded_rows += (uint64_t)(b->nb - n);
@@ -325,7 +375,7 @@ void completer_main(b2_tts_server *s) {
                 total += (size_t)r.nbytes;
                 d->recs.push_back(r);
             }
-            nlive += (t[1] > t[0] || t[2]) ? 1 : 0;
+            nlive += (t[1] > t[0] || t[2] == 1) ? 1 : 0;          // a cancelled row (ended 2) took no step
         }
         d->bytes.resize(total);
         size_t k = 0;
@@ -384,6 +434,7 @@ b2_tts_server *b2_tts_server_create(b2_ctx *c, b2_enc *enc, b2_dec *dec, int law
     s->st.capacity = (uint64_t)s->cap; s->st.depth = (uint64_t)depth;
     if (s->cap < 1) { set_error("b2_tts_server_create: the context's workspace holds no session of %d frames", NFRAMES); delete s; return nullptr; }
     s->slots.resize((size_t)s->nslots);
+    s->row_of.resize((size_t)s->nslots);
     for (int i = s->nslots - 1; i >= 0; i--) s->free_slots.push_back(i);
     const size_t S = (size_t)s->nslots, R = (size_t)s->cap, A = (size_t)s->adm_cap, Lm = (size_t)s->max_len;
     auto dal = [](auto **p, size_t n) { return cudaMalloc((void **)p, n * sizeof(**p)) == cudaSuccess; };
@@ -393,12 +444,13 @@ b2_tts_server *b2_tts_server_create(b2_ctx *c, b2_enc *enc, b2_dec *dec, int law
               dal(&s->d_idx, S) && dal(&s->d_ends, S) && dal(&s->d_minlen, S) && dal(&s->d_maxlen, S) && dal(&s->d_live, S) &&
               dal(&s->d_ids, A * Lm) && dal(&s->d_len, A) && dal(&s->d_adm, 3 * A) && dal(&s->d_rows, R) && dal(&s->d_dslots, R) &&
               dal(&s->d_tslots, R) && dal(&s->d_spk, A * SPK) && dal(&s->d_enc, A * Lm * 768) && dal(&s->d_mel, R * NFRAMES * NMEL) &&
-              dal(&s->d_prob, R * NSTEPS * 2) && cudaMemset(s->d_live, 0, S * sizeof(int32_t)) == cudaSuccess &&
+              dal(&s->d_prob, R * NSTEPS * 2) && dal(&s->d_can, 2 * R) && dal(&s->d_mark, R) &&
+              cudaMemset(s->d_live, 0, S * sizeof(int32_t)) == cudaSuccess && cudaMemset(s->d_mark, 0, R * sizeof(int32_t)) == cudaSuccess &&
               cudaMemset(s->d_mel, 0, R * NFRAMES * NMEL * sizeof(float)) == cudaSuccess;
     for (int i = 0; ok && i < depth; i++) {
         Call *b = new Call();
         s->calls_pool.push_back(b);
-        ok = hal(&b->h_ids, A * Lm) && hal(&b->h_len, A) && hal(&b->h_adm, 3 * A) && hal(&b->h_rows, R) && hal(&b->h_tri, 3 * R) &&
+        ok = hal(&b->h_ids, A * Lm) && hal(&b->h_len, A) && hal(&b->h_adm, 3 * A) && hal(&b->h_rows, R) && hal(&b->h_tri, 3 * R) && hal(&b->h_can, 2 * R) &&
              hal(&b->h_spk, A * SPK) && hal(&b->h_out, R * NBYTES) && dal(&b->d_out, R * NBYTES) && dal(&b->d_tri, 3 * R) &&
              cudaEventCreateWithFlags(&b->ev_c, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&b->ev_out, cudaEventDisableTiming) == cudaSuccess;
@@ -432,7 +484,8 @@ void b2_tts_server_destroy(b2_tts_server *s) {
     if (s->s_out) cudaStreamSynchronize(s->s_out);
     for (Call *b : s->calls_pool) {
         for (auto &kv : b->graphs) cudaGraphExecDestroy(kv.second.first);
-        for (void *p : {(void *)b->h_ids, (void *)b->h_len, (void *)b->h_adm, (void *)b->h_rows, (void *)b->h_tri, (void *)b->h_spk, (void *)b->h_out})
+        for (void *p : {(void *)b->h_ids, (void *)b->h_len, (void *)b->h_adm, (void *)b->h_rows, (void *)b->h_tri, (void *)b->h_can, (void *)b->h_spk,
+                        (void *)b->h_out})
             if (p) cudaFreeHost(p);
         if (b->d_out) cudaFree(b->d_out);
         if (b->d_tri) cudaFree(b->d_tri);
@@ -442,7 +495,7 @@ void b2_tts_server_destroy(b2_tts_server *s) {
     }
     for (void *p : {(void *)s->d_idx, (void *)s->d_ends, (void *)s->d_minlen, (void *)s->d_maxlen, (void *)s->d_live, (void *)s->d_ids, (void *)s->d_len,
                     (void *)s->d_adm, (void *)s->d_rows, (void *)s->d_dslots, (void *)s->d_tslots, (void *)s->d_spk, (void *)s->d_enc, (void *)s->d_mel,
-                    (void *)s->d_prob})
+                    (void *)s->d_prob, (void *)s->d_can, (void *)s->d_mark})
         if (p) cudaFree(p);
     for (Done *d : s->done_q) delete d;
     if (s->s_c) cudaStreamDestroy(s->s_c);
@@ -488,6 +541,51 @@ int b2_tts_server_submit(b2_tts_server *s, const int32_t *h_ids, const int32_t *
         s->cv_drive.notify_all();
     }
     return 0;
+}
+
+int b2_tts_server_cancel(b2_tts_server *s, const uint64_t *tags, int n) {
+    if (!s) return -set_error("null server");
+    if (n < 0 || (n > 0 && !tags)) return -set_error("b2_tts_server_cancel: null tags or n < 0");
+    const int64_t t_now = now_ns();
+    std::vector<uint64_t> want(tags, tags + n);
+    std::sort(want.begin(), want.end());
+    auto wanted = [&](uint64_t t) { return std::binary_search(want.begin(), want.end(), t); };
+    std::lock_guard<std::mutex> lk(s->mu);
+    if (s->stop) return -set_error("b2_tts_server_cancel: the server has stopped%s%s", s->async_error.empty() ? "" : ": ", s->async_error.c_str());
+    // pending sentences were never admitted: they leave the queue and get their last record now
+    Done *d = nullptr;
+    size_t w = 0;
+    for (size_t i = 0; i < s->pending.size(); i++) {
+        Pending &p = s->pending[i];
+        if (!wanted(p.tag)) {
+            if (w != i) s->pending[w] = std::move(p);
+            w++;
+            continue;
+        }
+        if (!d) d = new Done();
+        b2_tts_chunk r = {};
+        r.tag = p.tag; r.call = -1; r.admit_call = -1; r.t_submit_ns = p.t_submit; r.t_done_ns = t_now; r.ended = 2;
+        d->recs.push_back(r);
+    }
+    s->pending.resize(w);
+    const int npend = d ? (int)d->recs.size() : 0;
+    if (d) {
+        s->done_q.push_back(d);
+        s->unfinished -= npend;
+        s->st.ended += (uint64_t)npend;
+    }
+    // admitted sentences: the device decides in the next call (build_call), since a call in flight may end them first
+    int nlive = 0;
+    for (int sl : s->live_list) {
+        SlotInfo &si = s->slots[(size_t)sl];
+        if (!si.live || si.cancelled || !wanted(si.tag)) continue;
+        si.cancelled = true;
+        s->cancels.emplace_back(sl, si.seq);
+        nlive++;
+    }
+    if (npend) { s->cv_submit.notify_all(); s->cv_poll.notify_all(); }
+    if (nlive) s->cv_drive.notify_all();
+    return npend + nlive;
 }
 
 int b2_tts_server_poll(b2_tts_server *s, b2_tts_chunk *out, int max_out, uint8_t *h_g711, size_t g711_capacity, int timeout_ms) {

@@ -4,6 +4,7 @@ plus the fused tail.  torch is used only for device memory and streams."""
 from __future__ import annotations
 
 import ctypes
+import operator
 from typing import Dict, Optional, Sequence, Tuple
 
 import torch
@@ -627,9 +628,31 @@ class TTSServer:
         tags_a = (ctypes.c_uint64 * n)(*tg)
         _lib.check(self.lib.b2_tts_server_submit(h, ids_t.data_ptr(), lens_t.data_ptr(), n, sp_t.data_ptr(), tags_a), "tts_server_submit")
 
+    def cancel(self, tags) -> int:
+        """Cancels every sentence submitted with one of `tags` (one unsigned 64-bit tag or a sequence of them) whose last record has not been
+        made: the barge-in of TTSSndDispatch.cancel().  A pending sentence gets its last record at once (call -1, never admitted); an admitted
+        one at the next engine call, unless a call already in flight ends it first.  Records of calls in flight still arrive with their bytes.
+        A cancelled sentence's last record has nbytes 0 and `cancelled` True.  Returns the number of sentences found; unknown tags, sentences
+        that have ended and repeated cancels count 0."""
+        try:
+            tg = [operator.index(tags)]
+        except TypeError:
+            try:
+                tg = [operator.index(t) for t in tags]
+            except TypeError:
+                raise RuntimeError("tags must be unsigned 64-bit integers") from None
+        if any(not 0 <= t < 2 ** 64 for t in tg):
+            raise RuntimeError("tags must be unsigned 64-bit integers")
+        h = self._handle()
+        n = self.lib.b2_tts_server_cancel(h, (ctypes.c_uint64 * len(tg))(*tg), len(tg))
+        if n < 0:
+            raise RuntimeError("infernos_b200 tts_server_cancel: " + self.lib.b2_last_error(None).decode())
+        return n
+
     def poll(self, timeout_ms: int = 0):
-        """-> list of (record, bytes): record a dict with tag, call, admit_call, nbytes, ended, t_submit_ns, t_done_ns; bytes the G.711
-        payload of that sentence in that call.  timeout_ms: 0 = do not wait, < 0 = wait for the next completed call."""
+        """-> list of (record, bytes): record a dict with tag, call, admit_call, nbytes, ended, cancelled, t_submit_ns, t_done_ns; bytes the
+        G.711 payload of that sentence in that call.  `ended` marks a sentence's last record; `cancelled` one that cancel() ended.
+        timeout_ms: 0 = do not wait, < 0 = wait for the next completed call."""
         h = self._handle()
         n = self.lib.b2_tts_server_poll(h, self._recs, self._cap, self._bytes.data_ptr(), self._bytes.numel(), int(timeout_ms))
         if n < 0:
@@ -638,6 +661,7 @@ class TTSServer:
         raw = self._bytes.numpy()
         for r in self._recs[:n]:
             rec = {k: int(getattr(r, k)) for k, _ in _TTSChunk._fields_ if k != "g711_offset"}
+            rec["cancelled"] = rec["ended"] == 2
             rec["ended"] = bool(rec["ended"])
             out.append((rec, raw[r.g711_offset:r.g711_offset + r.nbytes].tobytes()))
         return out
